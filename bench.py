@@ -17,7 +17,12 @@ rank) is measured in the same run and reported as `extra.c3`.  C2 / C3 / C4 as -
 rank ("weak").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2|C3|C4|C4mf|C5] [--path fp32|tensor]
+                    [--dump-outputs DIR]
     python bench.py --impl reference ...     # CPU restatement of the reference (oracle port) on host cores
+
+--dump-outputs DIR writes what the last timed step of the headline workload returned (loss, loss ground truth, the
+residual sums, the parameter gradient, its norm, the parameter norm) and the parameters it left behind, one float32
+DIR/<name>.npy each.  Inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -162,9 +167,19 @@ def build_problem(w, device, seed=1):
     return drift_kind, drift, true, cov_half, model, params, opt
 
 
-def measure(name, args, shard, device, local_rank, steps, warmup, with_clocks):
+def dump_outputs(out_dir, out, params):
+    """The outputs of one hot-path step as out_dir/<name>.npy (float32): every tensor of the step's result dict and the
+    flat parameter vector after its optimizer update.  Copied to the host at once: later steps reuse these buffers."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = dict(out, params=params)
+    for key, t in arrays.items():
+        np.save(os.path.join(out_dir, key.replace(" ", "_") + ".npy"), t.detach().float().cpu().numpy())
+
+
+def measure(name, args, shard, device, local_rank, steps, warmup, with_clocks, dump_dir=None):
     """Warm-up + timed steps + e2e + per-kernel phases of one workload on this rank; returns the result dict (rank 0)
-    after the max-over-ranks reduction of the times."""
+    after the max-over-ranks reduction of the times.  dump_dir: where rank 0 writes the outputs of the last timed step."""
     from pde_inverse_problem_b200 import _lib as L
     from pde_inverse_problem_b200 import ops
     from pde_inverse_problem_b200.pipeline import HotPath, HotPathConfig
@@ -226,6 +241,8 @@ def measure(name, args, shard, device, local_rank, steps, warmup, with_clocks):
     t_dev = e0.elapsed_time(e1) / 1e3
     loss = float(out["loss"])
     assert math.isfinite(loss), "loss is not finite (a timed-out tcgen05 phase poisons it with NaN)"
+    if dump_dir is not None and shard.rank == 0:
+        dump_outputs(dump_dir, out, model.flat(params))
 
     # ---- e2e: ensemble in pinned host memory, H2D per chunk + D2H of the loss inside the timed region ----
     z0_host = torch.empty((n, 2 * d), dtype=torch.float32, pin_memory=True)
@@ -234,9 +251,8 @@ def measure(name, args, shard, device, local_rank, steps, warmup, with_clocks):
     hp.step(z0_host, seed=50, n_global=n_global, particle_offset=offset)  # warm the staging path
     barrier()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e2e_steps = max(1, min(steps, 3))
     f0.record()
-    for i in range(e2e_steps):
+    for i in range(steps):
         o = hp.step(z0_host, seed=2000 + i, n_global=n_global, particle_offset=offset)
         result_host[0].copy_(o["loss"], non_blocking=True)
         result_host[1].copy_(o["grad_norm"], non_blocking=True)
@@ -299,8 +315,8 @@ def measure(name, args, shard, device, local_rank, steps, warmup, with_clocks):
                                 % (3 * d * s_emit * cfg.chunk * 4 / 1e9)},
         "residual_evals_per_s": evals * steps / t_dev,
         "loss": loss,
-        "e2e": {"value": psteps * e2e_steps / t_e2e, "unit": "particle-steps/s",
-                "h2d_bytes_per_step": n * 2 * d * 4, "d2h_bytes_per_step": 8, "ms_per_step": t_e2e / e2e_steps * 1e3},
+        "e2e": {"value": psteps * steps / t_e2e, "unit": "particle-steps/s",
+                "h2d_bytes_per_step": n * 2 * d * 4, "d2h_bytes_per_step": 8, "ms_per_step": t_e2e / steps * 1e3},
         "gpu_launches": launches,
         "clocks": clocks,
         "roofline": ({"kernel": res_kernel, "bound": "hbm", "achieved": res_rate * 3 * d * 4 / 1e9, "peak": pk["hbm"],
@@ -334,11 +350,12 @@ def run_ours(args):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local_rank)
     device = torch.device("cuda", local_rank)
-    line = measure(args.workload, args, shard, device, local_rank, args.steps, args.warmup, with_clocks=True)
+    line = measure(args.workload, args, shard, device, local_rank, args.steps, args.warmup, with_clocks=True,
+                   dump_dir=args.dump_outputs)
     extra = None
     if args.workload == "C5" and not args.particles and not args.no_extra:
         # the C3 step (BASELINE.json configs[2], 2^22 particles per rank) in the same run
-        c3 = measure("C3", args, shard, device, local_rank, steps=max(3, min(args.steps, 5)), warmup=3, with_clocks=False)
+        c3 = measure("C3", args, shard, device, local_rank, args.steps, args.warmup, with_clocks=False)
         if c3 is not None:
             extra = {k: c3[k] for k in ("value", "unit", "ms_per_step", "scaling", "config", "residual_evals_per_s", "e2e",
                                         "roofline", "kernels", "steps", "warmup")}
@@ -462,7 +479,13 @@ def main():
                     help="residual kernel: tensor = tcgen05 bf16 GEMM path (rtol 1e-2, default), fp32 = CUDA-core parity path (rtol 1e-5)")
     ap.add_argument("--particles", type=int, default=0, help="override particles per rank")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":

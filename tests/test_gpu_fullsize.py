@@ -131,3 +131,25 @@ def test_pipeline_c5_shape_tensor_integrator_matches_fp32(cuda):
     assert relmax(stc[L.SUM_LOSS], s32[L.SUM_LOSS]) < 1e-2
     assert relmax(stc[L.SUM_GT], s32[L.SUM_GT]) < 1e-2
     assert relmax(gtc, g32) < 1e-2
+
+
+def test_bench_dumps_the_outputs_of_its_last_timed_step(cuda, tmp_path):
+    """bench.py --dump-outputs DIR: the result of the last of exactly --steps timed steps, one float32 .npy per output
+    (its loss is the loss of the JSON line), and the parameters that step left behind."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "C3", "--particles", "8192",
+                        "--steps", "2", "--warmup", "3", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600, cwd=root)
+    assert r.returncode == 0, r.stderr[-2000:]
+    j = json.loads(r.stdout)
+    assert j["steps"] == 2
+    names = {"loss", "loss_ground_truth", "sums", "grad", "grad_norm", "params_norm", "params"}
+    assert {f[:-4] for f in os.listdir(tmp_path)} == names
+    a = {k: np.load(tmp_path / (k + ".npy")) for k in names}
+    assert all(v.dtype == np.float32 and np.isfinite(v).all() for v in a.values())
+    assert float(a["loss"]) == j["loss"]
+    assert a["grad"].shape == a["params"].shape == (8 * 32 + 32 + 32 * 32 + 32 + 32 * 40 + 40,)
