@@ -131,6 +131,30 @@ int pdeip_kl_integrate_path(const float* z0, float* z_last, float* traj, float* 
                             int schedule, int state_layout, int traj_layout,
                             int emit_every, int emit_offset, int emit_drift, int path, void* stream);
 
+/* K1 with grad U = grad V_theta of a hypothesis model (model_kind / params / hidden / layers / n_gaussian exactly as
+ * in pdeip_model_eval and the residual kernels).  Every other argument, output, layout, schedule, Philox stream and
+ * emit_drift contract is that of pdeip_kl_integrate_path: the reference's underdamped_langevin_dynamics_scan driven by
+ * jax.grad of a fitted net.apply (utils/sampling_utils.py:25-52 with potential_grad = grad V_theta).
+ *   PDEIP_MODEL_MLP       hidden == 32 (narrower nets zero-padded), 1 <= layers <= 8, d <= 32; fp32 on the CUDA cores
+ *                         (rtol 1e-5 class).  PDEIP_PATH_TENSOR with layers == 2, d = 8, 16 or 32, Philox noise, REFERENCE
+ *                         schedule, AOS state, emit_every 1 and either traj == NULL (terminal state only, n arbitrary) or
+ *                         a PDEIP_TRAJ_BLOCK128 / PDEIP_TRAJ_TIME_SOA trajectory with emit_drift: the six GEMMs of a step
+ *                         (primal chain and input-gradient chain) run on tcgen05 with bf16 hi + lo split operands ("bf16
+ *                         GEMM path", rtol 1e-2 class); every other call takes the fp32 kernel (PDEIP_NO_TC_INTEGRATOR=1
+ *                         forces it);
+ *   PDEIP_MODEL_GMM       learned centres, sigma = 1: exactly pdeip_kl_integrate_path(PDEIP_DRIFT_GMM, params,
+ *                         n_gaussian, 1.0f, ...) on all of its kernels (bit-identical);
+ *   PDEIP_MODEL_QUADRATIC V = y.(yK + b): grad V = (K + K^T) y + b, fp32 on both paths.
+ * Rejected before any CUDA call: unknown model kind, NULL params (PDEIP_ERR_INVALID_ARG), d > 32, layers outside
+ * [1, 8], hidden != 32 (PDEIP_ERR_UNSUPPORTED), GMM with n_gaussian < 1 (PDEIP_ERR_INVALID_ARG). */
+int pdeip_kl_integrate_model(const float* z0, float* z_last, float* traj, float* tau,
+                             int64_t n_particles, int d, int n_steps, float dt, float gamma,
+                             int model_kind, const float* params, int hidden, int layers, int n_gaussian,
+                             const float* noise, const float* tau0,
+                             uint64_t seed, uint64_t particle_offset, uint32_t step_offset,
+                             int schedule, int state_layout, int traj_layout,
+                             int emit_every, int emit_offset, int emit_drift, int path, void* stream);
+
 /* Mean-field drift (interacting system, README.md:54-62): the ensemble mean on the common time grid obeys
  *   pbar' = (1 - gamma dt) pbar + sqrt(2 dt) xibar_s,  qbar' = qbar + dt pbar'   (the interaction cancels in the mean),
  * xibar_s = mean over ALL particles of the step-s Philox normals.  noise_sums accumulates (atomically, caller zeroes)

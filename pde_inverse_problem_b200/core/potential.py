@@ -87,3 +87,33 @@ class GMMPotential(Potential):
 
     def drift_spec(self):
         return L.DRIFT_GMM, self.mus, int(self.mus.shape[0]), self.sigma
+
+
+class ModelPotential(Potential):
+    """The potential V_theta of a fitted hypothesis model: `net` is a core.model model (V_hypothesis /
+    V_parametric_GMM / V_parametric_quadratic), `params` its parameter tree.  What the reference gets from
+    jax.grad(lambda x: net.apply(params, x)[0]): passing `ModelPotential(net, params).gradient` as `potential_grad`
+    to utils.sampling_utils.underdamped_langevin_dynamics_scan integrates the particles under the fitted drift
+    (pdeip_kl_integrate_model).
+
+    The parameter tree is held by reference and its flat buffer is looked up at every call.  The trainer updates
+    params["_flat"] in place, so one instance follows the fit; copy the tree to freeze a snapshot."""
+
+    def __init__(self, net, params):
+        self.net = net
+        self.params = params
+        self.dim = net.spec.d
+
+    def value(self, x):
+        if x.ndim == 1:
+            return self.net.apply(self.params, x)[0]
+        return self.net.apply(self.params, x)
+
+    def gradient(self, x):
+        if x.ndim == 1:
+            return self.net.gradient(self.params, x[None].contiguous())[0]
+        return self.net.gradient(self.params, x)
+
+    def drift_spec(self):
+        """(ModelSpec, flat parameter buffer) of pdeip_kl_integrate_model."""
+        return self.net.spec, self.net.flat(self.params)

@@ -5,11 +5,15 @@
 //   LINEAR   : grad U = A x  (kinetic OU tilde_F x, example_problems/kinetic_fokker_planck_example_OU.py:15-20;
 //              QuadraticPotential.gradient with mu = 0, core/potential.py:20-24)
 //   MEANFIELD: grad U = A (x - xbar)  (README.md:54-71)
+//   AFFINE   : grad U = M x + b  (the quadratic hypothesis model V = y.(yK + b): M = K + K^T,
+//              example_problems/kinetic_fokker_planck_example_OU.py:209-220)
+//   MLP      : grad U = grad V_theta of the hypothesis MLP (core/model.py:51-62), mlp_thread.cuh
 // Parameters live in shared memory, zero-padded to the compile-time width DP, so a runtime
 // d <= DP needs no masking inside the arithmetic (padded components stay exactly zero).
 #pragma once
 
 #include "common.cuh"
+#include "mlp_thread.cuh"
 
 namespace pdeip {
 
@@ -87,6 +91,36 @@ __device__ __forceinline__ void linear_grad_thread(const float (&x)[DP], const f
     for (int k = 0; k < DP; ++k) s = fmaf(A_s[i * DP + k], y[k], s);
     g[i] = s;
   }
+}
+
+// M_s: smem [DP][DP] row-major (padded), b_s: [DP];  g = M x + b
+template <int DP>
+__device__ __forceinline__ void affine_grad_thread(const float (&x)[DP], const float* __restrict__ M_s,
+                                                   const float* __restrict__ b_s, float (&g)[DP]) {
+#pragma unroll
+  for (int i = 0; i < DP; ++i) {
+    float s = 0.0f;
+#pragma unroll
+    for (int k = 0; k < DP; ++k) s = fmaf(M_s[i * DP + k], x[k], s);
+    g[i] = s + b_s[i];
+  }
+}
+
+// grad V_theta(x) of the hypothesis MLP, weights in smem (flat layout of pdeip.h, hidden width 32);
+// g[i] = 0 for d <= i < DP.  The per-point activations live in the thread's local memory.
+template <int DP, int LHMAX>
+__device__ __forceinline__ void mlp_grad_thread(const float (&x)[DP], const MlpShape<32>& sh,
+                                                const float* __restrict__ w_s, float (&g)[DP]) {
+  PointState<32, LHMAX> st;
+  MlpThread<32, LHMAX> net(sh, w_s, st);
+#pragma unroll
+  for (int i = 0; i < DP; ++i)
+    if (i < sh.d) st.x[i] = x[i];
+  net.primal_forward();
+  float gl[kDMax];
+  net.input_gradient(gl);
+#pragma unroll
+  for (int i = 0; i < DP; ++i) g[i] = i < sh.d ? gl[i] : 0.0f;
 }
 
 }  // namespace pdeip

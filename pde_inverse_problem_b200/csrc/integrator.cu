@@ -91,7 +91,12 @@ __device__ __forceinline__ void emit_drift_vals(float* __restrict__ base, int la
   }
 }
 
-template <int DP, int DRIFT>
+// drift kinds of the hypothesis models (pdeip_kl_integrate_model), internal to this file
+constexpr int kDriftAffine = 100;  // quadratic model: grad V = (K + K^T) y + b, params = [K (d*d), b (d)]
+constexpr int kDriftMlp = 101;     // MLP model: grad V_theta, params = the flat MLP buffer (hidden width 32)
+
+// LHMAX: hidden layers the per-thread MLP state is sized for (kDriftMlp only)
+template <int DP, int DRIFT, int LHMAX = 0>
 __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a) {
   extern __shared__ __align__(16) float smem[];
   // stage the drift parameters (zero-padded to DP) in shared memory
@@ -109,8 +114,20 @@ __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a
     }
   } else if constexpr (DRIFT == PDEIP_DRIFT_GMM) {
     load_padded<DP>(smem, a.drift_params, a.n_gaussian, a.d, threadIdx.x, blockDim.x);
+  } else if constexpr (DRIFT == kDriftAffine) {  // M = K + K^T [DP][DP], then b [DP], zero padded
+    shift_s = smem + DP * DP;
+    const float* K = a.drift_params;
+    for (int idx = threadIdx.x; idx < DP * DP; idx += blockDim.x) {
+      const int i = idx / DP, k = idx - i * DP;
+      A_s[idx] = (i < a.d && k < a.d) ? K[i * a.d + k] + K[k * a.d + i] : 0.0f;
+    }
+    for (int i = threadIdx.x; i < DP; i += blockDim.x) shift_s[i] = i < a.d ? K[a.d * a.d + i] : 0.0f;
+  } else if constexpr (DRIFT == kDriftMlp) {
+    const int P = MlpShape<32>{a.d, a.layers}.num_params();
+    for (int i = threadIdx.x; i < P; i += blockDim.x) smem[i] = a.drift_params[i];
   }
   __syncthreads();
+  const MlpShape<32> mlp_shape{a.d, a.layers};
 
   const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (n >= a.n) return;
@@ -144,6 +161,10 @@ __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a
     float g[DP];
     if constexpr (DRIFT == PDEIP_DRIFT_GMM) {
       gmm_grad_thread<DP>(q, smem, a.n_gaussian, a.inv_sigma2, g);
+    } else if constexpr (DRIFT == kDriftAffine) {
+      affine_grad_thread<DP>(q, A_s, shift_s, g);
+    } else if constexpr (DRIFT == kDriftMlp) {
+      mlp_grad_thread<DP, LHMAX>(q, mlp_shape, smem, g);
     } else if constexpr (DRIFT == PDEIP_DRIFT_LINEAR || DRIFT == PDEIP_DRIFT_MEANFIELD || kTable) {
       linear_grad_thread<DP>(q, A_s, shift_s, g);
       if constexpr (kTable) {
@@ -195,6 +216,10 @@ __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a
     float g[DP];
     if constexpr (DRIFT == PDEIP_DRIFT_GMM) {
       gmm_grad_thread<DP>(q, smem, a.n_gaussian, a.inv_sigma2, g);
+    } else if constexpr (DRIFT == kDriftAffine) {
+      affine_grad_thread<DP>(q, A_s, shift_s, g);
+    } else if constexpr (DRIFT == kDriftMlp) {
+      mlp_grad_thread<DP, LHMAX>(q, mlp_shape, smem, g);
     } else if constexpr (DRIFT == PDEIP_DRIFT_LINEAR || DRIFT == PDEIP_DRIFT_MEANFIELD || kTable) {
       linear_grad_thread<DP>(q, A_s, shift_s, g);
     } else {
@@ -501,6 +526,26 @@ static int launch_integrate(const IntegrateArgs& a, int drift_kind, int path, cu
   return PDEIP_OK;
 }
 
+// K1 under a hypothesis model's potential: the generic kernel with the affine (quadratic model) or MLP drift; under
+// PDEIP_PATH_TENSOR the MLP drift of the tcgen05 kernel's envelope (integrator_mlp_tc.cu).
+template <int DP>
+static int launch_integrate_model(const IntegrateArgs& a, int model_kind, int path, cudaStream_t st) {
+  if (model_kind == PDEIP_MODEL_MLP && path == PDEIP_PATH_TENSOR && integrate_mlp_tensor_ok(a))
+    return launch_integrate_mlp_tensor(a, st);
+  const unsigned grid = (unsigned)((a.n + 127) / 128);
+  if (model_kind == PDEIP_MODEL_QUADRATIC) {
+    kl_integrate_kernel<DP, kDriftAffine><<<grid, 128, sizeof(float) * (DP * DP + DP), st>>>(a);
+  } else {
+    // at most 9 768 floats (d = 32, 8 layers): below the 48 KB of shared memory a launch gets without opt-in
+    const size_t smem = sizeof(float) * (size_t)MlpShape<32>{a.d, a.layers}.num_params();
+    if (a.layers <= 2) kl_integrate_kernel<DP, kDriftMlp, 2><<<grid, 128, smem, st>>>(a);
+    else if (a.layers <= 4) kl_integrate_kernel<DP, kDriftMlp, 4><<<grid, 128, smem, st>>>(a);
+    else kl_integrate_kernel<DP, kDriftMlp, 8><<<grid, 128, smem, st>>>(a);
+  }
+  PDEIP_LAUNCH_OK();
+  return PDEIP_OK;
+}
+
 // ------------------------------------------------------------------------------------------
 // noise dumps (what the integrator draws in Philox mode) and the Gaussian initial ensemble
 // ------------------------------------------------------------------------------------------
@@ -646,13 +691,11 @@ __global__ void gaussian_sample_kernel(float* out, int64_t n, int dim, const flo
 
 using namespace pdeip;
 
-extern "C" int pdeip_kl_integrate_path(const float* z0, float* z_last, float* traj, float* tau,
-                                       int64_t n_particles, int d, int n_steps, float dt, float gamma,
-                                       int drift_kind, const float* drift_params, int n_gaussian, float sigma,
-                                       const float* noise, const float* tau0, uint64_t seed,
-                                       uint64_t particle_offset, uint32_t step_offset, int schedule,
-                                       int state_layout, int traj_layout, int emit_every, int emit_offset,
-                                       int emit_drift, int path, void* stream) {
+// validates the arguments common to every K1 entry point and fills the argument block
+static int integrate_args(IntegrateArgs& a, const float* z0, float* z_last, float* traj, float* tau,
+                          int64_t n_particles, int d, int n_steps, float dt, float gamma, const float* noise,
+                          const float* tau0, uint64_t seed, uint64_t particle_offset, uint32_t step_offset, int schedule,
+                          int state_layout, int traj_layout, int emit_every, int emit_offset, int emit_drift, int path) {
   PDEIP_REQUIRE(path == PDEIP_PATH_FP32 || path == PDEIP_PATH_TENSOR, PDEIP_ERR_INVALID_ARG, "unknown path %d", path);
   PDEIP_REQUIRE(z0 != nullptr, PDEIP_ERR_INVALID_ARG, "z0 is NULL");
   PDEIP_REQUIRE(n_particles >= 0 && d >= 1 && d <= 32, PDEIP_ERR_UNSUPPORTED,
@@ -668,15 +711,9 @@ extern "C" int pdeip_kl_integrate_path(const float* z0, float* z_last, float* tr
                 "PDEIP_TRAJ_BLOCK128 needs n_particles %% 128 == 0 (got %lld)", (long long)n_particles);
   PDEIP_REQUIRE(emit_every >= 1 && emit_offset >= 0 && emit_offset < emit_every, PDEIP_ERR_INVALID_ARG,
                 "emit_every/emit_offset out of range");
-  PDEIP_REQUIRE(drift_kind == PDEIP_DRIFT_NONE || drift_params != nullptr, PDEIP_ERR_INVALID_ARG,
-                "drift_params is NULL");
-  PDEIP_REQUIRE(drift_kind != PDEIP_DRIFT_GMM || (n_gaussian >= 1 && sigma > 0.0f), PDEIP_ERR_INVALID_ARG,
-                "GMM drift needs n_gaussian >= 1 and sigma > 0");
-  if (n_particles == 0) return PDEIP_OK;
-  IntegrateArgs a;
   a.z0 = z0; a.z_last = z_last; a.traj = traj; a.tau = tau; a.n = n_particles; a.d = d;
-  a.n_steps = n_steps; a.dt = dt; a.gamma = gamma; a.drift_params = drift_params;
-  a.n_gaussian = n_gaussian; a.inv_sigma2 = drift_kind == PDEIP_DRIFT_GMM ? 1.0f / (sigma * sigma) : 1.0f;
+  a.n_steps = n_steps; a.dt = dt; a.gamma = gamma; a.drift_params = nullptr;
+  a.n_gaussian = 0; a.inv_sigma2 = 1.0f; a.layers = 0;
   a.noise = noise; a.tau0 = tau0; a.seed = seed; a.particle_offset = particle_offset;
   a.step_offset = step_offset; a.schedule = schedule; a.state_layout = state_layout;
   a.traj_layout = traj_layout; a.emit_every = emit_every; a.emit_offset = emit_offset;
@@ -684,12 +721,74 @@ extern "C" int pdeip_kl_integrate_path(const float* z0, float* z_last, float* tr
   a.rk = philox_round_keys(seed);
   const int n_samples = n_steps;  // both schedules expose n_steps samples
   a.s_emit = (n_samples - emit_offset + emit_every - 1) / emit_every;
+  return PDEIP_OK;
+}
+
+extern "C" int pdeip_kl_integrate_path(const float* z0, float* z_last, float* traj, float* tau,
+                                       int64_t n_particles, int d, int n_steps, float dt, float gamma,
+                                       int drift_kind, const float* drift_params, int n_gaussian, float sigma,
+                                       const float* noise, const float* tau0, uint64_t seed,
+                                       uint64_t particle_offset, uint32_t step_offset, int schedule,
+                                       int state_layout, int traj_layout, int emit_every, int emit_offset,
+                                       int emit_drift, int path, void* stream) {
+  IntegrateArgs a;
+  const int rc = integrate_args(a, z0, z_last, traj, tau, n_particles, d, n_steps, dt, gamma, noise, tau0, seed,
+                                particle_offset, step_offset, schedule, state_layout, traj_layout, emit_every,
+                                emit_offset, emit_drift, path);
+  if (rc != PDEIP_OK) return rc;
+  PDEIP_REQUIRE(drift_kind == PDEIP_DRIFT_NONE || drift_params != nullptr, PDEIP_ERR_INVALID_ARG,
+                "drift_params is NULL");
+  PDEIP_REQUIRE(drift_kind != PDEIP_DRIFT_GMM || (n_gaussian >= 1 && sigma > 0.0f), PDEIP_ERR_INVALID_ARG,
+                "GMM drift needs n_gaussian >= 1 and sigma > 0");
+  if (n_particles == 0) return PDEIP_OK;
+  a.drift_params = drift_params;
+  a.n_gaussian = n_gaussian; a.inv_sigma2 = drift_kind == PDEIP_DRIFT_GMM ? 1.0f / (sigma * sigma) : 1.0f;
   cudaStream_t st = (cudaStream_t)stream;
   if (d <= 2) return launch_integrate<2>(a, drift_kind, path, st);
   if (d <= 4) return launch_integrate<4>(a, drift_kind, path, st);
   if (d <= 8) return launch_integrate<8>(a, drift_kind, path, st);
   if (d <= 16) return launch_integrate<16>(a, drift_kind, path, st);
   return launch_integrate<32>(a, drift_kind, path, st);
+}
+
+extern "C" int pdeip_kl_integrate_model(const float* z0, float* z_last, float* traj, float* tau,
+                                        int64_t n_particles, int d, int n_steps, float dt, float gamma,
+                                        int model_kind, const float* params, int hidden, int layers, int n_gaussian,
+                                        const float* noise, const float* tau0, uint64_t seed,
+                                        uint64_t particle_offset, uint32_t step_offset, int schedule,
+                                        int state_layout, int traj_layout, int emit_every, int emit_offset,
+                                        int emit_drift, int path, void* stream) {
+  PDEIP_REQUIRE(model_kind == PDEIP_MODEL_MLP || model_kind == PDEIP_MODEL_GMM || model_kind == PDEIP_MODEL_QUADRATIC,
+                PDEIP_ERR_INVALID_ARG, "unknown model kind %d", model_kind);
+  PDEIP_REQUIRE(params != nullptr, PDEIP_ERR_INVALID_ARG, "params is NULL");
+  PDEIP_REQUIRE(d >= 1 && d <= 32, PDEIP_ERR_UNSUPPORTED, "integrator supports 1 <= d <= 32 (got d=%d)", d);
+  if (model_kind == PDEIP_MODEL_GMM) {
+    // the parametric GMM model (learned centres, sigma = 1) is exactly the GMM drift, on all of its kernels
+    PDEIP_REQUIRE(n_gaussian >= 1, PDEIP_ERR_INVALID_ARG, "GMM model needs n_gaussian >= 1 (got %d)", n_gaussian);
+    return pdeip_kl_integrate_path(z0, z_last, traj, tau, n_particles, d, n_steps, dt, gamma, PDEIP_DRIFT_GMM, params,
+                                   n_gaussian, 1.0f, noise, tau0, seed, particle_offset, step_offset, schedule,
+                                   state_layout, traj_layout, emit_every, emit_offset, emit_drift, path, stream);
+  }
+  if (model_kind == PDEIP_MODEL_MLP) {
+    PDEIP_REQUIRE(hidden == 32, PDEIP_ERR_UNSUPPORTED,
+                  "MLP drift is built for hidden_dim == 32 (pad smaller widths with zeros); got %d", hidden);
+    PDEIP_REQUIRE(layers >= 1 && layers <= 8, PDEIP_ERR_UNSUPPORTED, "MLP drift supports 1 <= layers <= 8 (got %d)",
+                  layers);
+  }
+  IntegrateArgs a;
+  const int rc = integrate_args(a, z0, z_last, traj, tau, n_particles, d, n_steps, dt, gamma, noise, tau0, seed,
+                                particle_offset, step_offset, schedule, state_layout, traj_layout, emit_every,
+                                emit_offset, emit_drift, path);
+  if (rc != PDEIP_OK) return rc;
+  if (n_particles == 0) return PDEIP_OK;
+  a.drift_params = params;
+  a.layers = model_kind == PDEIP_MODEL_MLP ? layers : 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (d <= 2) return launch_integrate_model<2>(a, model_kind, path, st);
+  if (d <= 4) return launch_integrate_model<4>(a, model_kind, path, st);
+  if (d <= 8) return launch_integrate_model<8>(a, model_kind, path, st);
+  if (d <= 16) return launch_integrate_model<16>(a, model_kind, path, st);
+  return launch_integrate_model<32>(a, model_kind, path, st);
 }
 
 extern "C" int pdeip_kl_integrate(const float* z0, float* z_last, float* traj, float* tau,

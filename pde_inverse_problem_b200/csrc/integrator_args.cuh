@@ -21,6 +21,7 @@ struct IntegrateArgs {
   const float* drift_params;
   int n_gaussian;
   float inv_sigma2;
+  int layers;  // hidden layers of the MLP hypothesis model (pdeip_kl_integrate_model)
   const float* noise;
   const float* tau0;
   uint64_t seed;
@@ -39,5 +40,9 @@ struct IntegrateArgs {
 // integrator_tc.cu: GMM drift on the tensor cores (PDEIP_PATH_TENSOR)
 bool integrate_tensor_ok(const IntegrateArgs& a, int drift_kind);
 int launch_integrate_tensor(const IntegrateArgs& a, cudaStream_t st);
+
+// integrator_mlp_tc.cu: MLP (32 x 2) drift on the tensor cores (PDEIP_PATH_TENSOR of pdeip_kl_integrate_model)
+bool integrate_mlp_tensor_ok(const IntegrateArgs& a);
+int launch_integrate_mlp_tensor(const IntegrateArgs& a, cudaStream_t st);
 
 }  // namespace pdeip

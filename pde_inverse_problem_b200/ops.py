@@ -46,25 +46,15 @@ def _f32(t: Optional[torch.Tensor], name: str, allow_none: bool = False) -> Opti
 # ------------------------------------------------------------------------------------------------
 # K1 integrator
 # ------------------------------------------------------------------------------------------------
-def kl_integrate(z0: torch.Tensor, n_steps: int, dt: float, gamma: float, drift_kind: int,
-                 drift_params: Optional[torch.Tensor] = None, n_gaussian: int = 0, sigma: float = 1.0,
-                 noise: Optional[torch.Tensor] = None, tau0: Optional[torch.Tensor] = None, seed: int = 0,
-                 particle_offset: int = 0, step_offset: int = 0, schedule: int = L.SCHEDULE_REFERENCE,
-                 state_layout: int = L.LAYOUT_AOS, traj_layout: int = L.TRAJ_PARTICLE_MAJOR,
-                 want_traj: bool = True, want_tau: bool = False, emit_every: int = 1, emit_offset: int = 0,
-                 traj_out: Optional[torch.Tensor] = None, z_last_out: Optional[torch.Tensor] = None,
-                 emit_drift: bool = False, path: int = L.PATH_FP32,
-                 ) -> Tuple[torch.Tensor, Optional[torch.Tensor], Optional[torch.Tensor]]:
-    """pdeip_kl_integrate.  z0: [N,2d] (AOS) or [2d,N] (SOA).  Returns (z_last, traj|None, tau|None).
-    emit_drift: every trajectory sample is [x, v, grad U(x)] (3d components).
-    path: PATH_TENSOR runs the GMM drift contraction on tcgen05 where that kernel exists (see pdeip.h)."""
+def _k1_buffers(z0, n_steps, noise, tau0, schedule, state_layout, traj_layout, want_traj, want_tau, emit_every,
+                emit_offset, traj_out, z_last_out, emit_drift):
+    """Checked inputs and the outputs of one K1 call: (z0, n, d, noise, tau0, z_last, traj|None, tau|None)."""
     z0 = _f32(z0, "z0")
     if state_layout == L.LAYOUT_AOS:
         n, two_d = z0.shape
     else:
         two_d, n = z0.shape
     d = two_d // 2
-    drift_params = _f32(drift_params, "drift_params", allow_none=True)
     noise = _f32(noise, "noise", allow_none=True)
     tau0 = _f32(tau0, "tau0", allow_none=True)
     n_draws = n_steps + 1 if schedule == L.SCHEDULE_REFERENCE else n_steps
@@ -88,9 +78,54 @@ def kl_integrate(z0: torch.Tensor, n_steps: int, dt: float, gamma: float, drift_
         else:
             traj = torch.empty(shape, device=z0.device, dtype=torch.float32)
     tau = torch.empty((n, n_steps), device=z0.device, dtype=torch.float32) if want_tau else None
+    return z0, n, d, noise, tau0, z_last, traj, tau
+
+
+def kl_integrate(z0: torch.Tensor, n_steps: int, dt: float, gamma: float, drift_kind: int,
+                 drift_params: Optional[torch.Tensor] = None, n_gaussian: int = 0, sigma: float = 1.0,
+                 noise: Optional[torch.Tensor] = None, tau0: Optional[torch.Tensor] = None, seed: int = 0,
+                 particle_offset: int = 0, step_offset: int = 0, schedule: int = L.SCHEDULE_REFERENCE,
+                 state_layout: int = L.LAYOUT_AOS, traj_layout: int = L.TRAJ_PARTICLE_MAJOR,
+                 want_traj: bool = True, want_tau: bool = False, emit_every: int = 1, emit_offset: int = 0,
+                 traj_out: Optional[torch.Tensor] = None, z_last_out: Optional[torch.Tensor] = None,
+                 emit_drift: bool = False, path: int = L.PATH_FP32,
+                 ) -> Tuple[torch.Tensor, Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """pdeip_kl_integrate.  z0: [N,2d] (AOS) or [2d,N] (SOA).  Returns (z_last, traj|None, tau|None).
+    emit_drift: every trajectory sample is [x, v, grad U(x)] (3d components).
+    path: PATH_TENSOR runs the GMM drift contraction on tcgen05 where that kernel exists (see pdeip.h)."""
+    z0, n, d, noise, tau0, z_last, traj, tau = _k1_buffers(
+        z0, n_steps, noise, tau0, schedule, state_layout, traj_layout, want_traj, want_tau, emit_every, emit_offset,
+        traj_out, z_last_out, emit_drift)
+    drift_params = _f32(drift_params, "drift_params", allow_none=True)
     _ops.kl_integrate(z0, z_last, traj, tau, n, d, n_steps, float(dt), float(gamma), drift_kind, drift_params,
                       n_gaussian, float(sigma), noise, tau0, as_i64(seed), as_i64(particle_offset), step_offset, schedule,
                       state_layout, traj_layout, emit_every, emit_offset, 1 if emit_drift else 0, path)
+    launch_counter["n"] += 1
+    return z_last, traj, tau
+
+
+def kl_integrate_model(z0: torch.Tensor, n_steps: int, dt: float, gamma: float, spec: "ModelSpec",
+                       params: torch.Tensor, noise: Optional[torch.Tensor] = None, tau0: Optional[torch.Tensor] = None,
+                       seed: int = 0, particle_offset: int = 0, step_offset: int = 0,
+                       schedule: int = L.SCHEDULE_REFERENCE, state_layout: int = L.LAYOUT_AOS,
+                       traj_layout: int = L.TRAJ_PARTICLE_MAJOR, want_traj: bool = True, want_tau: bool = False,
+                       emit_every: int = 1, emit_offset: int = 0, traj_out: Optional[torch.Tensor] = None,
+                       z_last_out: Optional[torch.Tensor] = None, emit_drift: bool = False, path: int = L.PATH_FP32,
+                       ) -> Tuple[torch.Tensor, Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """pdeip_kl_integrate_model: kl_integrate with grad U = grad V_theta of the hypothesis model `spec` at the flat
+    parameters `params` (the buffer model_eval takes).  Same outputs and keyword arguments as kl_integrate;
+    emit_drift carries grad V_theta(x) of every emitted sample."""
+    z0, n, d, noise, tau0, z_last, traj, tau = _k1_buffers(
+        z0, n_steps, noise, tau0, schedule, state_layout, traj_layout, want_traj, want_tau, emit_every, emit_offset,
+        traj_out, z_last_out, emit_drift)
+    params = _f32(params, "params")
+    if d != spec.d or params.numel() != spec.num_params:
+        raise PdeipError(f"shape mismatch: the state has d={d}, params has {params.numel()} entries (expected "
+                         f"d={spec.d}, {spec.num_params} params)")
+    _ops.kl_integrate_model(z0, z_last, traj, tau, n, d, n_steps, float(dt), float(gamma), spec.kind, params,
+                            spec.hidden, spec.layers, spec.n_gaussian, noise, tau0, as_i64(seed),
+                            as_i64(particle_offset), step_offset, schedule, state_layout, traj_layout, emit_every,
+                            emit_offset, 1 if emit_drift else 0, path)
     launch_counter["n"] += 1
     return z_last, traj, tau
 

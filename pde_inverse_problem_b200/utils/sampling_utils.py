@@ -10,13 +10,15 @@ from .. import ops
 
 
 def drift_spec(potential_grad):
-    """Map the `potential_grad` callable the reference passes (Potential.gradient, GMM.py:120) to a drift
-    kind + parameter tensor of the C ABI."""
+    """Map the `potential_grad` callable the reference passes (Potential.gradient, GMM.py:120) to the drift of the
+    C ABI: (drift kind, parameter tensor, n_gaussian, sigma) for an analytic Potential, (ModelSpec, flat parameters)
+    for a core.potential.ModelPotential (a fitted hypothesis model)."""
     owner = getattr(potential_grad, "__self__", None)
     if owner is None or not hasattr(owner, "drift_spec"):
         raise NotImplementedError(
-            "potential_grad must be the .gradient method of a pde_inverse_problem_b200.core.potential.Potential; "
-            "arbitrary Python callables cannot run inside the fused CUDA integrator")
+            "potential_grad must be the .gradient method of a pde_inverse_problem_b200.core.potential.Potential "
+            "(GMMPotential, LinearPotential, QuadraticPotential, VoidPotential, or ModelPotential(net, params) for a "
+            "fitted model's grad V_theta); arbitrary Python callables cannot run inside the fused CUDA integrator")
     return owner.drift_spec()
 
 
@@ -24,14 +26,19 @@ def underdamped_langevin_dynamics_scan(q0_p0: torch.Tensor, n_steps: int, dt: fl
                                        gamma_friction: float, *, noise: Optional[torch.Tensor] = None,
                                        tau0: Optional[torch.Tensor] = None, particle_offset: int = 0,
                                        traj_layout: int = L.TRAJ_PARTICLE_MAJOR, want_trajectory: bool = True,
+                                       path: int = L.PATH_FP32,
                                        ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
     """Returns (last_sample [N,2d], trajectory [N,n_steps,2d], tau_trajectory [N,n_steps]) exactly like the
     vmapped reference (sampling_utils.py:52).  `key` is an integer seed (the reference passes one jax key
     per particle; here the per-particle stream is Philox(seed, particle_offset + n)).  `noise`/`tau0` inject
-    the random draws for parity runs."""
-    kind, params, n_gaussian, sigma = drift_spec(potential_grad)
-    z_last, traj, tau = ops.kl_integrate(
-        q0_p0, n_steps, float(dt), float(gamma_friction), kind, params, n_gaussian=n_gaussian, sigma=sigma,
-        noise=noise, tau0=tau0, seed=int(key), particle_offset=particle_offset,
-        schedule=L.SCHEDULE_REFERENCE, traj_layout=traj_layout, want_traj=want_trajectory, want_tau=True)
-    return z_last, traj, tau
+    the random draws for parity runs.  `path`: the kernel path of pdeip_kl_integrate_path (see pdeip.h)."""
+    spec = drift_spec(potential_grad)
+    common = dict(noise=noise, tau0=tau0, seed=int(key), particle_offset=particle_offset,
+                  schedule=L.SCHEDULE_REFERENCE, traj_layout=traj_layout, want_traj=want_trajectory, want_tau=True,
+                  path=path)
+    if isinstance(spec[0], ops.ModelSpec):
+        model_spec, flat = spec
+        return ops.kl_integrate_model(q0_p0, n_steps, float(dt), float(gamma_friction), model_spec, flat, **common)
+    kind, params, n_gaussian, sigma = spec
+    return ops.kl_integrate(q0_p0, n_steps, float(dt), float(gamma_friction), kind, params, n_gaussian=n_gaussian,
+                            sigma=sigma, **common)
