@@ -6,8 +6,9 @@
 //
 // Organisation.  One CTA per SM, persistent over 128-point tiles; NS tiles ("slots") are in flight per CTA so
 // that one slot's epilogue hides the other's GEMM hand-off latency (NS = 2 for d <= 8, 1 otherwise).
-//   * 8 epilogue warps: thread = (point row == TMEM lane, 16 of the 32 units / 24 of the 48 outputs); 1 MMA warp:
-//     one elected lane issues every tcgen05.mma of both slots.
+//   * epilogue warps: thread = (point row == TMEM lane, one part of the units; Team): 16 warps in the one-slot kernels
+//     (8 of the 32 hidden units, 8 + 2 of the 40 outputs), 8 in the two-slot kernel (16 / 24); 1 MMA warp: one elected
+//     lane issues every tcgen05.mma of both slots.
 //   * operands: bf16 in shared memory, no-swizzle core-matrix layout (umma.cuh); every tile is written once and
 //     used K-major (layer GEMMs, points x units) and through the transposed view (batch-reduced dW GEMMs).
 //     Weights and the input x are split hi + lo (two bf16 terms), activations are rounded to bf16 once.
@@ -21,7 +22,7 @@
 //   * dW_l = t^T zbar0 + a1^T zbar1 + c^T za^ accumulates over ALL tiles of the CTA in persistent TMEM
 //     columns: each term is an M = 128 GEMM over the 128 points whose A operand is the transposed view of the
 //     activation tile started at the band of that stream ("band-shifted accumulate"): rows 0..31 of D are the
-//     wanted 32 x N block, rows >= 32 are never read.  db_l = sum_p zbar0 is kept in registers.
+//     wanted 32 x N block, rows >= 32 are never read.  db_l = sum_p zbar0 is kept per row (registers, or TMEM: C_DB).
 //   phases  P0 z0,z1_0 | P1 z1,z1_1,z2^_1 | P2 u,u1,u2^ | P3 aa2, ab1_2 (+dW2: a1) | P4 aa1, ab1_1 (+dW1: a1) |
 //           P5 g (+dW0: v) | P6 zg^_0 | P7 zg^_1 | P8 ug^ | P9 ab_2, aa2 (+dW2: t, c) | P10 ab_1, aa1 (+dW1: t, c) |
 //           P11 (dW0: x_hi, x_lo, g^).   E_k = epilogue between P_{k-1} and P_k.
@@ -78,6 +79,10 @@ constexpr uint32_t C_AB1 = C_R + 48, C_AA1R = C_R + 96;                     // P
 // MMA warp on the uniform datapath the GEMM phases shorten by ~100 cycles each: d = 32 2.055e9 -> 2.24e9 evals/s.
 constexpr uint32_t C_AOP = C_SLOT0 + SLOT_COLS;  // [312, 360): columns = 4 x (chunk index within the operand)
 constexpr uint32_t C_AOPX = C_AOP + 48;           // [360, 408): the A operands of P0 ([x_hi | x_lo], v) when E0 runs a tile ahead (PIPE_X)
+// [408, 512): one-slot kernels keep the per-row bias-gradient sums here, 26 per epilogue part (db0 8, db1 8, db2 10):
+// db0 at [408 + 8 part, +8), db1 at [440 + 8 part, +8), db2 chunk units at [472 + 8 part, +8), db2 pair at [504 + 2 part, +2)
+constexpr uint32_t C_DB = C_AOPX + 48;
+static_assert(C_DB + 4 * 26 == 512, "TMEM column map");
 
 // ---- shared memory ---------------------------------------------------------------------------------------------
 // Z tile chunk map (24 chunks of 8 columns)
@@ -85,6 +90,26 @@ constexpr int ZC_ZA2 = 0, ZC_ZA1 = 6, ZC_ZA0 = 10, ZC_TA = 14, ZC_TB = 20;
 // A tile chunk map (12 chunks): t | a1 (later the g-stream operand ag^) | a2^ (later c = a2^ + ag^)
 constexpr int AC_T = 0, AC_A1 = 4, AC_C = 8;
 
+// Thread shape.  Epilogue thread = (point row == TMEM lane, one "part" of the units): warp w reads TMEM lane quadrant
+// q = w & 3 and owns part w >> 2.  One-slot kernels run 16 epilogue warps (4 parts: 8 of the 32 hidden units, and of
+// the 40 output units 8 + 2, see OutCols), the two-slot kernel 8 (2 parts: 16 hidden units, 24 of the 48 output
+// columns): with one slot nothing overlaps an epilogue phase, so its length is the tile's critical path, and it is
+// bound by the latency of each thread's dependent chain, which more warps per scheduler shorten.
+template <int NS>
+struct Team {
+  static constexpr int kEpiWarps = NS == 1 ? 16 : 8;
+  static constexpr int kParts = kEpiWarps / 4;
+  static constexpr int kEpiThreads = 32 * kEpiWarps;
+  static constexpr int kThreads = kEpiThreads + 32;  // + one MMA-issuing warp (threads taking part in the named barriers)
+  // Launched with a full extra warpgroup (the MMA warp and three idle warps) so that `setmaxnreg` can move registers:
+  // the register file is 16 K per scheduler and each scheduler hosts kEpiWarps / 4 epilogue warps and one warp of the
+  // extra group; the extra group shrinks and the epilogue groups grow (Regs<NS> below; no spills).
+  static constexpr int kLaunchThreads = kEpiThreads + 128;
+  // registers per thread the kernel is compiled and launched at (__launch_bounds__(kLaunchThreads, 1): the register
+  // file over the threads, rounded down to the allocation granule of 8); tests/test_residual_tc_resources.py checks
+  // that ptxas reports exactly this
+  static constexpr int kLaunchRegs = 65536 / kLaunchThreads / 8 * 8;
+};
 template <int DP, int NS>
 struct Cfg {
   static constexpr int XC = DP / 8;                  // chunks per input band
@@ -132,8 +157,10 @@ struct Cfg {
 #define PDEIP_TC_STAGE 0
 #endif
   static constexpr uint32_t STAGE_BYTES = (PDEIP_TC_STAGE && NS == 1) ? 128u * 3u * DP * 4u : 0u;
+  // one-slot kernels: the five loss sums of every epilogue thread, [5][epilogue threads] floats (see kSumsSmem)
+  static constexpr uint32_t SUMS_BYTES = NS == 1 ? 5u * 4u * Team<NS>::kEpiThreads : 0u;
   static constexpr uint32_t O_TRUE = O_BIAS + 512, O_MISC = O_TRUE + TP_BYTES, O_STAGE = O_MISC + 128,
-                            TOTAL = O_STAGE + STAGE_BYTES;
+                            O_SUMS = O_STAGE + STAGE_BYTES, TOTAL = O_SUMS + SUMS_BYTES;
   static_assert(TOTAL <= 227u * 1024u && O_STAGE % 128 == 0 && O_X2 % 1024 == 0, "shared-memory budget");
 };
 
@@ -152,15 +179,9 @@ struct Cfg {
 #ifndef PDEIP_TC_LO_FWD
 #define PDEIP_TC_LO_FWD true  // lo halves of W1, W2 in the forward layer GEMMs P1, P2
 #endif
-constexpr int kEpiThreads = 256;            // 8 epilogue warps: thread = (point row, 16-unit half of a 32-unit tile)
-constexpr int kThreads = kEpiThreads + 32;  // + one MMA-issuing warp (threads taking part in the named barriers)
-// Launched with a full third warpgroup (three idle warps) so that `setmaxnreg` can move registers: the register file
-// is 16 K per scheduler and each scheduler hosts two epilogue warps and one warp of the third group; the kernel is
-// compiled for 168 registers, the third group shrinks and the epilogue groups grow (Regs<NS> below; no spills).
-constexpr int kLaunchThreads = 384;
-// (epilogue, third group) register budgets after setmaxnreg (the kernel is compiled and launched at 168)
+// (epilogue, extra group) register budgets after setmaxnreg
 #ifndef PDEIP_TC_REGS1_EPI
-#define PDEIP_TC_REGS1_EPI 232
+#define PDEIP_TC_REGS1_EPI 104
 #define PDEIP_TC_REGS1_MMA 40
 #endif
 #ifndef PDEIP_TC_REGS2_EPI
@@ -171,9 +192,12 @@ template <int NS>
 struct Regs {
   static constexpr int kEpi = NS == 2 ? PDEIP_TC_REGS2_EPI : PDEIP_TC_REGS1_EPI;
   static constexpr int kMma = NS == 2 ? PDEIP_TC_REGS2_MMA : PDEIP_TC_REGS1_MMA;
-  // measured: only the registers released by the third group's warp are available to the two epilogue warps of a
-  // scheduler (2 x 216 + 80 = 512 never returns; 2 x 208 + 88 works)
-  static_assert(2 * (kEpi - 168) <= 168 - kMma && kEpi % 8 == 0 && kMma % 8 == 0 && kMma >= 24 && kEpi <= 256,
+  // measured: a scheduler's epilogue warps can only grow into what its warp of the extra group releases, i.e. the
+  // pool is (epilogue warps per scheduler + 1) x the launch count (two-slot kernel at 168: 2 x 216 + 80 = 512 never
+  // returns; 2 x 208 + 88 = 504 works).  One-slot kernels at 96: 4 x 104 + 40 = 456 <= 480; 4 x 112 + 40 does not fit.
+  static constexpr int kEpiPerSched = Team<NS>::kEpiWarps / 4, kLaunch = Team<NS>::kLaunchRegs;
+  static_assert(kEpiPerSched * kEpi + kMma <= (kEpiPerSched + 1) * kLaunch && kEpi >= kLaunch && kMma <= kLaunch &&
+                    kEpi % 8 == 0 && kMma % 8 == 0 && kMma >= 24 && kEpi <= 256,
                 "setmaxnreg budgets: an impossible request never returns (the kernel hangs)");
 };
 
@@ -209,17 +233,24 @@ constexpr int kTraceTiles = 64;
 #else
 #define TC_PROBE(id, unit0, arr, n) do { } while (0)
 #endif
+// the output-layer units of this thread (OutCols oc)
+#define TC_PROBE_OUT(id, arr)                                                                       \
+  do {                                                                                              \
+    TC_PROBE(id, oc.unit0(), arr, 8 * OutCols<NP>::NC);                                             \
+    if constexpr (OutCols<NP>::PAIR) TC_PROBE(id, oc.pair_unit(), (arr) + 8 * OutCols<NP>::NC, 2); \
+  } while (0)
 
 // epilogue side: operands written -> visible to the tensor core; TMEM accesses ordered; signal the MMA warp
-template <bool PROXY_FENCE = true>
+template <int NS, bool PROXY_FENCE = true>
 __device__ __forceinline__ void epi_arrive(int slot) {
   if constexpr (PROXY_FENCE) fence_async_smem();
   fence_before_sync();
-  asm volatile("bar.arrive %0, %1;" ::"r"(1 + slot), "n"(kThreads) : "memory");
+  asm volatile("bar.arrive %0, %1;" ::"r"(1 + slot), "n"(Team<NS>::kThreads) : "memory");
 }
 // MMA warp: wait until every epilogue thread has arrived
+template <int NS>
 __device__ __forceinline__ void mma_wait_operands(int slot) {
-  asm volatile("bar.sync %0, %1;" ::"r"(1 + slot), "n"(kThreads) : "memory");
+  asm volatile("bar.sync %0, %1;" ::"r"(1 + slot), "n"(Team<NS>::kThreads) : "memory");
   fence_after_sync();
 }
 
@@ -430,21 +461,42 @@ __device__ __forceinline__ void tm_st4(uint32_t taddr, const uint32_t* r) {
                "r"(r[2]), "r"(r[3])
                : "memory");
 }
-// NU fp32 columns (NU = 16 or 24) -> floats, no wait
+__device__ __forceinline__ void tm_ld2(uint32_t taddr, uint32_t* r) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0,%1}, [%2];" : "=r"(r[0]), "=r"(r[1]) : "r"(taddr) : "memory");
+}
+__device__ __forceinline__ void tm_ld1(uint32_t taddr, uint32_t* r) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(r[0]) : "r"(taddr) : "memory");
+}
+__device__ __forceinline__ void tm_st2(uint32_t taddr, const uint32_t* r) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1,%2};" ::"r"(taddr), "r"(r[0]), "r"(r[1]) : "memory");
+}
+__device__ __forceinline__ void tm_st1(uint32_t taddr, uint32_t r) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x1.b32 [%0], {%1};" ::"r"(taddr), "r"(r) : "memory");
+}
+// NU fp32 columns (NU = 8, 16 or 24) -> floats, no wait
 template <int NU>
 __device__ __forceinline__ void tm_ldf(uint32_t taddr, float* v) {
   uint32_t* r = reinterpret_cast<uint32_t*>(v);
-  tm_ld16(taddr, r);
-  if constexpr (NU == 24) tm_ld8(taddr + 16, r + 16);
+  if constexpr (NU == 8) {
+    tm_ld8(taddr, r);
+  } else {
+    tm_ld16(taddr, r);
+    if constexpr (NU == 24) tm_ld8(taddr + 16, r + 16);
+  }
 }
 // NU parked values = NU / 2 columns of packed bf16 pairs
 template <int NU>
 __device__ __forceinline__ void tm_ldp(uint32_t taddr, uint32_t* r) {
-  tm_ld8(taddr, r);
-  if constexpr (NU == 24) tm_ld4(taddr + 8, r + 8);
+  if constexpr (NU == 8) {
+    tm_ld4(taddr, r);
+  } else {
+    tm_ld8(taddr, r);
+    if constexpr (NU == 24) tm_ld4(taddr + 8, r + 8);
+  }
 }
+// stores only (the caller waits with tm_wait_st)
 template <int NU>
-__device__ __forceinline__ void tm_park(uint32_t taddr, const float* v) {
+__device__ __forceinline__ void tm_park_st(uint32_t taddr, const float* v) {
   uint32_t r[NU / 2];
 #pragma unroll
   for (int i = 0; i < NU / 2; ++i) r[i] = pack2(v[2 * i], v[2 * i + 1]);
@@ -454,8 +506,63 @@ __device__ __forceinline__ void tm_park(uint32_t taddr, const float* v) {
     tm_st8(taddr, r);
     if constexpr (NU == 24) tm_st4(taddr + 8, r + 8);
   }
+}
+template <int NU>
+__device__ __forceinline__ void tm_park(uint32_t taddr, const float* v) {
+  tm_park_st<NU>(taddr, v);
   tm_wait_st();
 }
+
+// Output-layer units (48 columns, 40 real) of epilogue part `part` out of NP.  NP = 2: columns [24 part, +24).  NP = 4:
+// chunk `part` (columns [8 part, +8)) plus the pair 32 + 2 part, 33 + 2 part of chunk 4, 10 units per thread; chunk 5
+// (columns 40..47) is padding with zero weights and bias that no thread owns.  Every array over a thread's output units
+// holds the NC chunk units first, then the PAIR units.  Packed bf16 values (parked in TMEM or stored as an operand)
+// follow the same map: column pair k of the chunk units at word 4 NC part + k, the pair at word 16 + part.
+template <int NP>
+struct OutCols {
+  static constexpr int NC = NP == 2 ? 3 : 1;  // full 8-unit chunks per thread
+  static constexpr bool PAIR = NP == 4;
+  static constexpr int NU = 8 * NC + (PAIR ? 2 : 0);
+  const int part;
+  __device__ __forceinline__ int unit0() const { return 8 * NC * part; }  // first chunk unit
+  __device__ __forceinline__ int chunk0() const { return NC * part; }
+  __device__ __forceinline__ int pair_unit() const { return 32 + 2 * part; }
+  __device__ __forceinline__ int unit(int i) const { return i < 8 * NC ? unit0() + i : pair_unit() + i - 8 * NC; }
+  // NU fp32 accumulator columns of this thread (no wait)
+  __device__ __forceinline__ void ldf(uint32_t taddr, float* v) const {
+    tm_ldf<8 * NC>(taddr + unit0(), v);
+    if constexpr (PAIR) tm_ld2(taddr + pair_unit(), reinterpret_cast<uint32_t*>(v + 8 * NC));
+  }
+  // NU / 2 parked words (no wait)
+  __device__ __forceinline__ void ldp(uint32_t taddr, uint32_t* r) const {
+    tm_ldp<8 * NC>(taddr + 4 * NC * part, r);
+    if constexpr (PAIR) tm_ld1(taddr + 16 + part, r + 4 * NC);
+  }
+  __device__ __forceinline__ void park(uint32_t taddr, const float* v) const {
+    tm_park_st<8 * NC>(taddr + 4 * NC * part, v);
+    if constexpr (PAIR) tm_st1(taddr + 16 + part, pack2(v[8 * NC], v[8 * NC + 1]));
+    tm_wait_st();
+  }
+  // bias (or any 48-float vector in shared memory) of this thread's units
+  __device__ __forceinline__ void ld_smem(const float* b, float* v) const {
+#pragma unroll
+    for (int i = 0; i < 2 * NC; ++i)
+      *reinterpret_cast<float4*>(v + 4 * i) = *reinterpret_cast<const float4*>(b + unit0() + 4 * i);
+    if constexpr (PAIR) *reinterpret_cast<float2*>(v + 8 * NC) = *reinterpret_cast<const float2*>(b + pair_unit());
+  }
+  // this thread's units of a 48-column band of an operand tile (first chunk c0; `row` = the thread's row offset) and,
+  // with TS, of its A-operand copy in TMEM (first word w0 of the band in this thread's lane)
+  template <bool TS>
+  __device__ __forceinline__ void put(uint8_t* row, int c0, uint32_t w0, const float* v) const {
+#pragma unroll
+    for (int c = 0; c < NC; ++c) put_op<TS>(row, (c0 + NC * part + c) * 128, w0 + 4 * (NC * part + c), v + 8 * c);
+    if constexpr (PAIR) {
+      const uint32_t w = pack2(v[8 * NC], v[8 * NC + 1]);
+      *reinterpret_cast<uint32_t*>(row + (c0 + 4) * 128 + 4 * part) = w;
+      if constexpr (TS) tm_st1(w0 + 16 + part, w);
+    }
+  }
+};
 
 // inline true gradient (LINEAR: A x; GMM: core/potential.py:32-37), components [8 cg, 8 cg + 8) of point p (p < 0: none).
 // Cold path (tests and the reference-shaped API; the pipeline stores grad U next to the point): kept out of line.
@@ -534,7 +641,7 @@ __device__ __forceinline__ float2 bc2(float x) { return make_float2(x, x); }
 // carries none of the other modes' code (the epilogue is instruction-fetch sensitive).
 constexpr int kModeKfp0T = 0, kModeBnd = 1, kModeFp0T = 2;
 template <int DP, int NS, int MODE>
-__global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(const ResidualArgs a, int* status) {
+__global__ void __launch_bounds__(Team<NS>::kLaunchThreads, 1) mlp_residual_tc_kernel(const ResidualArgs a, int* status) {
   constexpr bool BND = MODE == kModeBnd, FPM = MODE == kModeFp0T;
 #ifndef PDEIP_TC_TS
 #define PDEIP_TC_TS 1  // see C_AOP above
@@ -558,11 +665,15 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
   constexpr bool kPipeX = Cfg<DP, NS>::PIPE_X;  // E0 / P0 of the next tile ride behind E10 / with P11 (see Cfg)
   constexpr bool kPipeFlow = kPipeX;  // the schedule that goes with the second buffer
   using S = Cfg<DP, NS>;
+  constexpr int kEpiThreads = Team<NS>::kEpiThreads, kThreads = Team<NS>::kThreads, kLaunchThreads = Team<NS>::kLaunchThreads;
+  constexpr int NP = Team<NS>::kParts;  // epilogue parts (see Team)
+  constexpr int UH = 32 / NP;           // hidden units per epilogue thread
+  constexpr int HC = UH / 8;            // ... in 8-unit chunks
   extern __shared__ __align__(1024) uint8_t sm[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const bool is_mma_warp = warp == kEpiThreads / 32;
   const int q = warp & 3;         // TMEM lane quadrant of this warp
-  const int half = (warp >> 2) & 1;  // which 16 units of a 32-unit tile (24 of a 48-unit tile) this thread owns
+  const int part = warp >> 2;      // which UH of the 32 hidden units (and which output units, OutCols) this thread owns
   const int row = q * 32 + lane;  // point within the tile == TMEM lane == operand tile row
   const int d = a.d;
   const MlpShape<H> sh{d, 2};
@@ -716,7 +827,7 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
             }
           };
           TC_TRACE_DECL_MMA;
-          mma_wait_operands(s);
+          mma_wait_operands<NS>(s);
           if (elect_one()) {
             TC_TRACE(4);
             switch (ph) {
@@ -896,13 +1007,38 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
 #ifdef PDEIP_TC_PROBE
     float* probe = reinterpret_cast<float*>(status) + 2048;
 #endif
-    // bias-gradient sums over this thread's row: units [16 half, +16) of the hidden layers, [24 half, +24) of the output
-    float db0[16], db1[16], db2[24];
+    const OutCols<NP> oc{part};
+    constexpr int UO = OutCols<NP>::NU;  // output units per thread
+    // bias-gradient sums over this thread's row: hidden units [UH part, +UH), output units of oc.  The two-slot kernel
+    // keeps them in registers.  One-slot kernels keep them in TMEM (C_DB; 104 registers per thread do not hold them next
+    // to the phase temporaries): E9, E10 and E11 load them with their other TMEM reads in front of the GEMM wait and store
+    // them with the operand stores that their hand-off waits for anyway.
+    constexpr bool kDbTmem = NS == 1;
+    static_assert(!kDbTmem || (UH == 8 && UO == 10), "C_DB map: 8 + 8 + 10 columns per part");
+    const uint32_t LDB = TB + ((uint32_t)(q * 32) << 16) + C_DB;
+    const uint32_t cdb0 = LDB + 8 * part, cdb1 = LDB + 32 + 8 * part, cdb2 = LDB + 64 + 8 * part, cdb2p = LDB + 96 + 2 * part;
+    auto db_ld = [&](uint32_t col, float* v) { tm_ld8(col, reinterpret_cast<uint32_t*>(v)); };
+    auto db_st = [&](uint32_t col, const float* v) { tm_st8(col, reinterpret_cast<const uint32_t*>(v)); };
+    auto db2_ld = [&](float* v) { db_ld(cdb2, v); tm_ld2(cdb2p, reinterpret_cast<uint32_t*>(v + 8)); };
+    auto db2_st = [&](const float* v) { db_st(cdb2, v); tm_st2(cdb2p, reinterpret_cast<const uint32_t*>(v + 8)); };
+    float db0[UH], db1[UH], db2[UO];
 #pragma unroll
-    for (int i = 0; i < 16; ++i) { db0[i] = 0.f; db1[i] = 0.f; }
+    for (int i = 0; i < UH; ++i) { db0[i] = 0.f; db1[i] = 0.f; }
 #pragma unroll
-    for (int i = 0; i < 24; ++i) db2[i] = 0.f;
+    for (int i = 0; i < UO; ++i) db2[i] = 0.f;
+    if constexpr (kDbTmem) {
+      db_st(cdb0, db0);
+      db_st(cdb1, db1);
+      db2_st(db2);
+      tm_wait_st();
+    }
+    // loss sums of this thread's row: registers in the two-slot kernel; one-slot kernels keep them in shared memory
+    // (S::O_SUMS, [k][thread]), read and written once per tile by E3 (d1, d2) and E6 (g2, gt2, gd2), as the db sums
+    constexpr bool kSumsSmem = NS == 1;
+    float* const sums_s = reinterpret_cast<float*>(sm + S::O_SUMS) + tid;
     float sum_g2 = 0.f, sum_gt2 = 0.f, sum_gd2 = 0.f, sum_d1 = 0.f, sum_d2 = 0.f;
+    if constexpr (kSumsSmem)
+      for (int k = 0; k < 5; ++k) sums_s[k * kEpiThreads] = 0.f;
     const float gamma = a.coef, gamma4 = 4.f * a.coef;
     const float cgw = 1.f / (float)fpd;  // coefficient of the |g|^2 term per row (FP: 1/d per direction row; else 1)
     const int dimw = (FPM ? d : 2 * d) + (a.tg.kind == PDEIP_DRIFT_IN_POINTS ? d : 0);  // floats per point
@@ -912,30 +1048,31 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
     const uint32_t offZ = (uint32_t)(row & 7) * 16u + (uint32_t)(row >> 3) * S::RG_Z;
     const uint32_t LA0 = TB + ((uint32_t)(q * 32) << 16) + C_SLOT0;
     const uint32_t LOP = TB + ((uint32_t)(q * 32) << 16) + C_AOP;  // this thread's lane of the A-operand columns (kTS)
-    const int u16 = 16 * half, u24 = 24 * half;  // first unit owned in 32- / 48-unit tiles
-    // prefetched input chunks: item j = half + 2 i;  j in [0, XC): x chunk j;  [XC, 2 XC): v;  [2 XC, 3 XC): stored gt
-    constexpr int NI = (3 * S::XC + 1) / 2;
+    const int uh = UH * part;  // first hidden unit owned
+    // prefetched input chunks: item j = part + NP i;  j in [0, XC): x chunk j;  [XC, 2 XC): v;  [2 XC, 3 XC): stored gt
+    constexpr int NI = (3 * S::XC + NP - 1) / NP;
     float xin0[NI][8], xin1[NI][8];
     // BLOCK128 point sets with d == DP (the pipeline's layout and the benchmark widths): the tile is one block of
     // [dimw][128] floats, so every component of this thread's row sits at a COMPILE-TIME offset from one base pointer:
     // 48 loads with immediate offsets at d = 32 instead of ~12 instructions of 64-bit index arithmetic per load (the
     // generic path below: 560 instructions and ~2.3 k cycles per tile in the phase trace).
     const bool fast_in = !FPM && a.layout == PDEIP_LAYOUT_BLOCK128 && d == DP;
-    auto load_into = [&](float (&xin)[NI][8], int64_t t, const int i0 = 0, const int i1 = 64) {  // items [i0, i1)
+    // items of the bands in `bands` (bit 0 x, bit 1 v, bit 2 stored gt)
+    auto load_into = [&](float (&xin)[NI][8], int64_t t, const int bands = 7) {
       if (fast_in) {
         const int64_t pp = t * 128 + row;
         const bool inside = t < n_tiles && pp < a.n_points;
-        // item j = half + 2 i holds components [8 j, 8 j + 8) of the row (band j / XC, chunk j % XC, DP = 8 XC): the
-        // runtime half goes into the base pointer, the rest is an immediate
-        const float* const pb = a.points + (inside ? t * (int64_t)(128 * dimw) + row : (int64_t)0) + half * (8 * 128);
+        // item j = part + NP i holds components [8 j, 8 j + 8) of the row (band j / XC, chunk j % XC, DP = 8 XC): the
+        // runtime part goes into the base pointer, the rest is an immediate
+        const float* const pb = a.points + (inside ? t * (int64_t)(128 * dimw) + row : (int64_t)0) + part * (8 * 128);
         const bool has_gt = a.tg.kind == PDEIP_DRIFT_IN_POINTS;
 #pragma unroll
         for (int i = 0; i < NI; ++i) {
-          if (i < i0 || i >= i1) continue;
-          if (half + 2 * i >= 3 * S::XC) continue;       // (d = 8: the fourth item does not exist)
-          if (half + 2 * i >= 2 * S::XC && !has_gt) continue;  // stored true gradient: only if the rows carry it
+          if (part + NP * i >= 3 * S::XC) continue;       // (d = 8: the fourth item does not exist)
+          if (!((bands >> ((part + NP * i) / S::XC)) & 1)) continue;
+          if (part + NP * i >= 2 * S::XC && !has_gt) continue;  // stored true gradient: only if the rows carry it
 #pragma unroll
-          for (int e = 0; e < 8; ++e) xin[i][e] = __ldg(pb + (16 * i + e) * 128);
+          for (int e = 0; e < 8; ++e) xin[i][e] = __ldg(pb + (8 * NP * i + e) * 128);
         }
         return;
       }
@@ -948,8 +1085,8 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
       const float* const pbase = a.points + point_base(a.layout, pc, dimw);
 #pragma unroll
       for (int i = 0; i < NI; ++i) {
-        if (i < i0 || i >= i1) continue;
-        const int j = half + 2 * i;
+        const int j = part + NP * i;
+        if (j < 3 * S::XC && !((bands >> (j / S::XC)) & 1)) continue;
         const int band = (j / S::XC) < 3 ? (j / S::XC) : 0, cg = j % S::XC;
         const int bandc = (band < 2 || a.tg.kind == PDEIP_DRIFT_IN_POINTS) ? band : 0;
         // FP rows hold [x (d), grad V_true (d, IN_POINTS)]: the gt band sits right after x, the v band is e_dir
@@ -978,9 +1115,9 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
     };
     if (use_stage && tid == 0) stage_issue(tile_begin);
     // two separate branches: each slot's loads target its own registers directly (no select on the loaded value)
-    auto load_inputs = [&](int s, int64_t t, const int i0 = 0, const int i1 = 64) {
-      if (NS == 2 && s == 1) load_into(xin1, t, i0, i1);
-      else load_into(xin0, t, i0, i1);
+    auto load_inputs = [&](int s, int64_t t, const int bands = 7) {
+      if (NS == 2 && s == 1) load_into(xin1, t, bands);
+      else load_into(xin0, t, bands);
     };
 #ifndef PDEIP_TC_L2_PREFETCH
 #define PDEIP_TC_L2_PREFETCH 1
@@ -993,11 +1130,11 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
     auto prefetch_inputs = [&](int64_t t) {
       if (FPM || t >= n_tiles || (t + 1) * 128 > a.n_points) return;  // FP tiles / ragged last tile: not worth a special case
       if (a.layout == PDEIP_LAYOUT_SOA) {  // dimw component segments of 512 B
-        if ((a.n_points & 3) == 0 && half == 0 && row < dimw)
+        if ((a.n_points & 3) == 0 && part == 0 && row < dimw)
           asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.points + (int64_t)row * a.n_points + t * 128),
                        "r"(512u)
                        : "memory");
-      } else if (half == 0 && row == 0) {  // AOS and BLOCK128: the tile is one contiguous block of 128 x dimw floats
+      } else if (part == 0 && row == 0) {  // AOS and BLOCK128: the tile is one contiguous block of 128 x dimw floats
         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.points + t * 128 * dimw),
                      "r"((uint32_t)(512 * dimw))
                      : "memory");
@@ -1017,7 +1154,7 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
     auto emit_x = [&](const float (&xin)[NI][8], const bool valid_t, uint8_t* const Xd) {
 #pragma unroll
       for (int i = 0; i < NI; ++i) {
-        const int j = half + 2 * i;
+        const int j = part + NP * i;
         const int band = j / S::XC, cg = j % S::XC;
         if (band == 0) {
           float hi[8], lo[8];
@@ -1079,7 +1216,12 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
       constexpr bool kEarlyLoads = true;  // (at d = 32 this used to spill; the shorter life of the input registers fixed that)
 #if PDEIP_TC_L2_PREFETCH
       if constexpr (ph == 0) {
-        if (!use_stage) load_inputs(s, tile);
+        if (!use_stage) load_inputs(s, tile, kPipeFlow ? 3 : 7);  // (PIPE_X: first tile only; stored gt below)
+      }
+      // PIPE_X: this tile's stored true gradient (an L2 hit since the prefetch in E4 one tile ago) for E6, read in front
+      // of E5's GEMM wait.  Read in E10 with x and v, its 8 registers would live across six phases and spill at d = 32.
+      if constexpr (kPipeFlow && ph == 5) {
+        if (a.tg.kind == PDEIP_DRIFT_IN_POINTS) load_inputs(s, tile, 4);
       }
 #endif
       if constexpr (kStage && ph == 0) {
@@ -1093,7 +1235,7 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
           const int dir = FPM ? (int)((uint32_t)tile % fpd) : -1;
 #pragma unroll
           for (int i = 0; i < NI; ++i) {
-            const int j = half + 2 * i;
+            const int j = part + NP * i;
             const int band = (j / S::XC) < 3 ? (j / S::XC) : 0, cg = j % S::XC;
             if (band < 2) {
 #pragma unroll
@@ -1114,19 +1256,19 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         // E1: t1, a1_1 = s1 z1, a2^_1 = t a1 z1      E2: t2, a1_2, a2^_2 = s1 z2^ + t a1 z1     (a2^ = -a2 / 2)
         constexpr bool l1 = ph == 1;
         uint8_t* const At = l1 ? A1 : A2;
-        float z0[16], z1[16], z2[16];
-        tm_ldf<16>(LA + (l1 ? C_Z0 : C_Z1) + u16, z0);
-        tm_ldf<16>(LA + (l1 ? C_Z10 : C_Z11) + u16, z1);
-        if constexpr (!l1) tm_ldf<16>(LA + C_Z21 + u16, z2);
-        float bb[16];
+        float z0[UH], z1[UH], z2[UH];
+        tm_ldf<UH>(LA + (l1 ? C_Z0 : C_Z1) + uh, z0);
+        tm_ldf<UH>(LA + (l1 ? C_Z10 : C_Z11) + uh, z1);
+        if constexpr (!l1) tm_ldf<UH>(LA + C_Z21 + uh, z2);
+        float bb[UH];
 #pragma unroll
-        for (int i = 0; i < 4; ++i)
-          *reinterpret_cast<float4*>(bb + 4 * i) = *reinterpret_cast<const float4*>(bias_s + (l1 ? 0 : 32) + u16 + 4 * i);
+        for (int i = 0; i < UH / 4; ++i)
+          *reinterpret_cast<float4*>(bb + 4 * i) = *reinterpret_cast<const float4*>(bias_s + (l1 ? 0 : 32) + uh + 4 * i);
         tm_wait_ld();
-        float t[16], s1[16], q1[16], q2[16];
+        float t[UH], s1[UH], q1[UH], q2[UH];
 #if PDEIP_TC_PACKED
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
+        for (int i = 0; i < UH / 2; ++i) {
           const float2 zb = __fadd2_rn(pr(z0, i), pr(bb, i));
           const float2 t2 = make_float2(tanh_fast(zb.x), tanh_fast(zb.y));
           const float2 s2 = __ffma2_rn(__fmul2_rn(t2, bc2(-1.f)), t2, bc2(1.f));
@@ -1138,7 +1280,7 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         }
 #else
 #pragma unroll
-        for (int i = 0; i < 16; ++i) {
+        for (int i = 0; i < UH; ++i) {
           t[i] = tanh_fast(z0[i] + bb[i]);
           s1[i] = fmaf(-t[i], t[i], 1.f);
           q1[i] = s1[i] * z1[i];
@@ -1147,36 +1289,34 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         }
 #endif
 #pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          put_op<kTS>(At, (AC_T + 2 * half + c) * 128, LOP + 4 * (AC_T + 2 * half + c), t + 8 * c);
-          put_op<kTS>(At, (AC_A1 + 2 * half + c) * 128, LOP + 4 * (AC_A1 + 2 * half + c), q1 + 8 * c);
-          put_op<kTS>(At, (AC_C + 2 * half + c) * 128, LOP + 4 * (AC_C + 2 * half + c), q2 + 8 * c);
+        for (int c = 0; c < HC; ++c) {
+          put_op<kTS>(At, (AC_T + HC * part + c) * 128, LOP + 4 * (AC_T + HC * part + c), t + 8 * c);
+          put_op<kTS>(At, (AC_A1 + HC * part + c) * 128, LOP + 4 * (AC_A1 + HC * part + c), q1 + 8 * c);
+          put_op<kTS>(At, (AC_C + HC * part + c) * 128, LOP + 4 * (AC_C + HC * part + c), q2 + 8 * c);
         }
-        tm_park<16>(LA + (l1 ? C_S1P1 : C_S1P2) + 8 * half, s1);
-        TC_PROBE(l1 ? 0 : 3, u16, t, 16);
-        TC_PROBE(l1 ? 1 : 4, u16, q1, 16);
-        TC_PROBE(l1 ? 2 : 5, u16, q2, 16);
+        tm_park<UH>(LA + (l1 ? C_S1P1 : C_S1P2) + UH / 2 * part, s1);
+        TC_PROBE(l1 ? 0 : 3, uh, t, UH);
+        TC_PROBE(l1 ? 1 : 4, uh, q1, UH);
+        TC_PROBE(l1 ? 2 : 5, uh, q2, UH);
       } else if constexpr (ph == 3) {
         // E3: za^2 = 8 u, s1v = -8 u1 + 4 gamma u, s0p = 8 u2^ + 4 gamma u1, D_v V, D_v^2 V
-        float u[24], u1[24], u2[24];
-        tm_ldf<24>(LA + C_U + u24, u);
-        tm_ldf<24>(LA + C_U1 + u24, u1);
-        tm_ldf<24>(LA + C_U2 + u24, u2);
-        float bb[24];
-#pragma unroll
-        for (int i = 0; i < 6; ++i)
-          *reinterpret_cast<float4*>(bb + 4 * i) = *reinterpret_cast<const float4*>(bias_s + 64 + u24 + 4 * i);
+        float u[UO], u1[UO], u2[UO];
+        oc.ldf(LA + C_U, u);
+        oc.ldf(LA + C_U1, u1);
+        oc.ldf(LA + C_U2, u2);
+        float bb[UO];
+        oc.ld_smem(bias_s + 64, bb);
         tm_wait_ld();
         // seeds of l = alpha D_v^2 V + beta D_v V (+ |g|^2):  0T set alpha = -2, beta = 2 gamma;  BND alpha = 0, beta = coef
         const float k8 = BND ? 0.f : 8.f * mk, kg = (BND ? 2.f * a.coef : gamma4) * mk;
         float d1 = 0.f, d2a = 0.f, d2b = 0.f;
-        float za[24], sv[24], sp[24];
+        float za[UO], sv[UO], sp[UO];
 #if PDEIP_TC_PACKED
         {
           float2 e1 = bc2(0.f), e2a = bc2(0.f), e2b = bc2(0.f);
           const float2 k82 = bc2(k8), nk82 = bc2(-k8), kg2 = bc2(kg);
 #pragma unroll
-          for (int i = 0; i < 12; ++i) {
+          for (int i = 0; i < UO / 2; ++i) {
             const float2 uu = __fadd2_rn(pr(u, i), pr(bb, i));
             const float2 v1 = pr(u1, i), v2 = pr(u2, i);
             e1 = __ffma2_rn(uu, v1, e1);
@@ -1190,7 +1330,7 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         }
 #else
 #pragma unroll
-        for (int i = 0; i < 24; ++i) {
+        for (int i = 0; i < UO; ++i) {
           const float uu = u[i] + bb[i];
           d1 = fmaf(uu, u1[i], d1);
           d2a = fmaf(u1[i], u1[i], d2a);
@@ -1200,42 +1340,47 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
           sp[i] = fmaf(k8, u2[i], kg * u1[i]);
         }
 #endif
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-          put_op<kTS>(Z, (ZC_ZA2 + 3 * half + c) * 128, LOP + 4 * (3 * half + c), za + 8 * c);
-          put_op<kTS>(Z, (ZC_TA + 3 * half + c) * 128, LOP + 24 + 4 * (3 * half + c), sv + 8 * c);
-        }
-        tm_park<24>(LA + C_S0P + 12 * half, sp);
+        oc.template put<kTS>(Z, ZC_ZA2, LOP, za);
+        oc.template put<kTS>(Z, ZC_TA, LOP + 24, sv);
+        oc.park(LA + C_S0P, sp);
         // this thread's share of D_v V = 2 u.u1 and D_v^2 V = 2 (u1.u1 + u.u2), u2 = -2 u2^
+        if constexpr (kSumsSmem) {
+          sum_d1 = sums_s[3 * kEpiThreads];
+          sum_d2 = sums_s[4 * kEpiThreads];
+        }
         sum_d1 = fmaf(2.f * mk, d1, sum_d1);
         sum_d2 = fmaf(mk, 2.f * d2a - 4.f * d2b, sum_d2);
-        TC_PROBE(6, u24, za, 24);
-        TC_PROBE(7, u24, sv, 24);
-        TC_PROBE(8, u24, sp, 24);
+        if constexpr (kSumsSmem) {
+          sums_s[3 * kEpiThreads] = sum_d1;
+          sums_s[4 * kEpiThreads] = sum_d2;
+        }
+        TC_PROBE_OUT(6, za);
+        TC_PROBE_OUT(7, sv);
+        TC_PROBE_OUT(8, sp);
       } else if constexpr (ph == 4 || ph == 5) {
-        if constexpr (kPipeFlow && ph == 4) prefetch_inputs(tile + tile_stride);  // read behind E10's hand-off
+        if constexpr (kPipeFlow && ph == 4) prefetch_inputs(tile + tile_stride);  // read in E10
         // E4 (hidden layer 2) / E5 (hidden layer 1):  aa^ = 4 aa from the GEMM of za^
         //   za^' = aa^ s1,  zbar1' = s1 ab1 + 2 t aa^ a1,  pz = a1 (aa^ a1 - 2 t ab1)
         constexpr bool l2 = ph == 4;
         const uint8_t* At = l2 ? A2 : A1;
-        float aa[16], ab1[16], t[16], a1[16];
-        uint32_t s1p[8];
-        tm_ldp<16>(LA + (l2 ? C_S1P2 : C_S1P1) + 8 * half, s1p);
+        float aa[UH], ab1[UH], t[UH], a1[UH];
+        uint32_t s1p[UH / 2];
+        tm_ldp<UH>(LA + (l2 ? C_S1P2 : C_S1P1) + UH / 2 * part, s1p);
 #pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          load_chunk(At, (AC_T + 2 * half + c) * 128, t + 8 * c);
-          load_chunk(At, (AC_A1 + 2 * half + c) * 128, a1 + 8 * c);
+        for (int c = 0; c < HC; ++c) {
+          load_chunk(At, (AC_T + HC * part + c) * 128, t + 8 * c);
+          load_chunk(At, (AC_A1 + HC * part + c) * 128, a1 + 8 * c);
         }
         tm_wait_ld();
         if constexpr (kEarlyLoads) wait_gemm();
-        tm_ldf<16>(LA + (l2 ? C_AA2 : C_AA1) + u16, aa);
-        tm_ldf<16>(LA + (l2 ? C_AB12 : C_AB11) + u16, ab1);
+        tm_ldf<UH>(LA + (l2 ? C_AA2 : C_AA1) + uh, aa);
+        tm_ldf<UH>(LA + (l2 ? C_AB12 : C_AB11) + uh, ab1);
         tm_wait_ld();
         TC_FINE(0);
-        float za[16], zb[16], pz[16];
+        float za[UH], zb[UH], pz[UH];
 #if PDEIP_TC_PACKED
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
+        for (int i = 0; i < UH / 2; ++i) {
           const float2 s2 = unp2(s1p, i), aa2 = pr(aa, i), a12 = pr(a1, i), ab2 = pr(ab1, i);
           const float2 tt = __fmul2_rn(pr(t, i), bc2(2.f));
           const float2 qq = __fmul2_rn(aa2, a12);
@@ -1245,7 +1390,7 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         }
 #else
 #pragma unroll
-        for (int i = 0; i < 16; ++i) {
+        for (int i = 0; i < UH; ++i) {
           const float s1 = unp(s1p, i);
           za[i] = aa[i] * s1;
           const float qq = aa[i] * a1[i];
@@ -1254,73 +1399,107 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         }
 #endif
 #pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          put_op<kTS>(Z, ((l2 ? ZC_ZA1 : ZC_ZA0) + 2 * half + c) * 128, LOP + 4 * (2 * half + c), za + 8 * c);
+        for (int c = 0; c < HC; ++c) {
+          put_op<kTS>(Z, ((l2 ? ZC_ZA1 : ZC_ZA0) + HC * part + c) * 128, LOP + 4 * (HC * part + c), za + 8 * c);
           // zbar1' is an A operand of P4; zbar1'' (E5) only feeds the dW0 chain (shared memory)
-          put_op<(kTS && l2)>(Z, ((l2 ? ZC_TB : ZC_TA) + 2 * half + c) * 128, LOP + 16 + 4 * (2 * half + c), zb + 8 * c);
+          put_op<(kTS && l2)>(Z, ((l2 ? ZC_TB : ZC_TA) + HC * part + c) * 128, LOP + 16 + 4 * (HC * part + c), zb + 8 * c);
         }
         TC_FINE(1);
-        tm_park<16>(LA + (l2 ? C_PZ2 : C_PZ1) + 8 * half, pz);
+        tm_park<UH>(LA + (l2 ? C_PZ2 : C_PZ1) + UH / 2 * part, pz);
         TC_FINE(2);
-        TC_PROBE(l2 ? 9 : 12, u16, za, 16);
-        TC_PROBE(l2 ? 10 : 13, u16, zb, 16);
-        TC_PROBE(l2 ? 11 : 14, u16, pz, 16);
+        TC_PROBE(l2 ? 9 : 12, uh, za, UH);
+        TC_PROBE(l2 ? 10 : 13, uh, zb, UH);
+        TC_PROBE(l2 ? 11 : 14, uh, pz, UH);
       } else if constexpr (ph == 6) {
         // E6: g^ = g / 2 band (the GEMM gives 4 g);  |g|^2, |g_true|^2, |g_true - g|^2
+        if constexpr (kSumsSmem) {
+          sum_g2 = sums_s[0];
+          sum_gt2 = sums_s[kEpiThreads];
+          sum_gd2 = sums_s[2 * kEpiThreads];
+        }
+        // which items carry the sums: the stored gt band, else the x band (gt from the true potential, or zero)
+        const bool gt_stored = a.tg.kind == PDEIP_DRIFT_IN_POINTS;
+        const float mkc = mk * cgw;  // FP: each of the d direction rows of a point carries 1/d of the per-point sums
+        auto add_sums = [&](const float* gv, const float* gt) {
+#pragma unroll
+          for (int e = 0; e < 8; ++e) {
+            const float df = gt[e] - gv[e];
+            sum_g2 = fmaf(mkc * gv[e], gv[e], sum_g2);
+            sum_gt2 = fmaf(mkc * gt[e], gt[e], sum_gt2);
+            sum_gd2 = fmaf(mkc * df, df, sum_gd2);
+          }
+        };
+        // g^ band first (the operand of the next GEMM), then the sums; the sums of the true-potential kinds come last, so
+        // that no input register is live across their out-of-line true_grad_chunk call (a call clobbers the caller-saved
+        // registers: at 104 registers the stored-gt items spilled around it)
+        auto g_chunk = [&](int cg, float* gv) {
+          tm_ld8(LA + C_G + 8 * cg, reinterpret_cast<uint32_t*>(gv));
+          tm_wait_ld();
+#pragma unroll
+          for (int e = 0; e < 8; ++e) gv[e] *= 0.25f;
+        };
 #pragma unroll
         for (int i = 0; i < NI; ++i) {
-          const int j = half + 2 * i;
+          const int j = part + NP * i;
           const int band = j / S::XC, cg = j % S::XC;
-          const bool own_sum = a.tg.kind == PDEIP_DRIFT_IN_POINTS ? band == 2 : band == 0;
-          if (j < 3 * S::XC && (band == 0 || own_sum)) {
-            float g4[8], gv[8], gt[8];
-            tm_ld8(LA + C_G + 8 * cg, reinterpret_cast<uint32_t*>(g4));
-            tm_wait_ld();
+          if (band == 0) {
+            float gv[8], gh[8];
+            g_chunk(cg, gv);
 #pragma unroll
-            for (int e = 0; e < 8; ++e) {
-              gv[e] = 0.25f * g4[e];
-              gt[e] = 0.f;
-            }
-            if (band == 0) {
-              float gh[8];
+            for (int e = 0; e < 8; ++e) gh[e] = (0.5f * cgw) * gv[e];  // the g-stream is linear in its direction: c_g g / 2
+            put_op<kTS>(X, (S::XC_G + cg) * 128, LOP + 4 * cg, gh);
+            TC_PROBE(15, cg * 8, gv, 8);
+          }
+        }
+        if (gt_stored) {
 #pragma unroll
-              for (int e = 0; e < 8; ++e) gh[e] = (0.125f * cgw) * g4[e];  // the g-stream is linear in its direction: c_g g / 2
-              put_op<kTS>(X, (S::XC_G + cg) * 128, LOP + 4 * cg, gh);
-              TC_PROBE(15, cg * 8, gv, 8);
-            }
-            if (own_sum) {
-              const float mkc = mk * cgw;  // FP: each of the d direction rows of a point carries 1/d of the per-point sums
-              if (a.tg.kind == PDEIP_DRIFT_IN_POINTS) {
-#pragma unroll
-                for (int e = 0; e < 8; ++e) {
-                  const int u = cg * 8 + e;
-                  float val;
-                  if (kStage && use_stage) val = stage[((FPM ? d : 2 * d) + (u < d ? u : 0)) * 128];  // still this tile's block
-                  else val = (NS == 2 && s == 1) ? xin1[i][e] : xin0[i][e];
-                  gt[e] = (valid && u < d) ? val : 0.f;
-                }
-              } else if (a.tg.kind == PDEIP_DRIFT_LINEAR || a.tg.kind == PDEIP_DRIFT_GMM) {
-                true_grad_chunk<DP>(a, tp, valid ? p : (int64_t)-1, dimw, cg, gt);
-              }
+          for (int i = 0; i < NI; ++i) {
+            const int j = part + NP * i;
+            const int band = j / S::XC, cg = j % S::XC;
+            if (j < 3 * S::XC && band == 2) {
+              float gv[8], gt[8];
+              g_chunk(cg, gv);
 #pragma unroll
               for (int e = 0; e < 8; ++e) {
-                const float df = gt[e] - gv[e];
-                sum_g2 = fmaf(mkc * gv[e], gv[e], sum_g2);
-                sum_gt2 = fmaf(mkc * gt[e], gt[e], sum_gt2);
-                sum_gd2 = fmaf(mkc * df, df, sum_gd2);
+                const int u = cg * 8 + e;
+                float val;
+                if (kStage && use_stage) val = stage[((FPM ? d : 2 * d) + (u < d ? u : 0)) * 128];  // still this tile's block
+                else val = (NS == 2 && s == 1) ? xin1[i][e] : xin0[i][e];
+                gt[e] = (valid && u < d) ? val : 0.f;
               }
+              add_sums(gv, gt);
             }
           }
+        } else {
+#pragma unroll
+          for (int i = 0; i < NI; ++i) {
+            const int j = part + NP * i;
+            const int band = j / S::XC, cg = j % S::XC;
+            if (band == 0) {
+              float gv[8], gt[8];
+              g_chunk(cg, gv);
+#pragma unroll
+              for (int e = 0; e < 8; ++e) gt[e] = 0.f;
+              if (a.tg.kind == PDEIP_DRIFT_LINEAR || a.tg.kind == PDEIP_DRIFT_GMM)
+                true_grad_chunk<DP>(a, tp, valid ? p : (int64_t)-1, dimw, cg, gt);
+              add_sums(gv, gt);
+            }
+          }
+        }
+        if constexpr (kSumsSmem) {
+          sums_s[0] = sum_g2;
+          sums_s[kEpiThreads] = sum_gt2;
+          sums_s[2 * kEpiThreads] = sum_gd2;
         }
       } else if constexpr (ph == 7 || ph == 8) {
         // E7: ag^_1 = s1_1 zg^_0 -> a1 band of A1;  c_1 = a2^_1 + ag^_1       E8: the same for hidden layer 2
         constexpr bool l1 = ph == 7;
         uint8_t* const At = l1 ? A1 : A2;
-        float zg[16], a2[16];
-        uint32_t s1p[8];
-        tm_ldp<16>(LA + (l1 ? C_S1P1 : C_S1P2) + 8 * half, s1p);
+        float zg[UH], a2[UH];
+        uint32_t s1p[UH / 2];
+        tm_ldp<UH>(LA + (l1 ? C_S1P1 : C_S1P2) + UH / 2 * part, s1p);
 #pragma unroll
-        for (int c = 0; c < 2; ++c) load_chunk(At, (AC_C + 2 * half + c) * 128, a2 + 8 * c);
+        for (int c = 0; c < HC; ++c) load_chunk(At, (AC_C + HC * part + c) * 128, a2 + 8 * c);
         tm_wait_ld();
         if constexpr (kEarlyLoads && !(kGram && l1)) wait_gemm();  // kGram: zg^_0 is a P5 result, already waited for in E6
         if constexpr (kStage && l1) {
@@ -1328,55 +1507,56 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
           // the proxy fence of that arrive): the next tile's block may overwrite it, five phases ahead of its E0
           if (use_stage && tid == 0) stage_issue(tile + tile_stride);
         }
-        tm_ldf<16>(LA + (l1 ? C_ZG0 : C_ZG1) + u16, zg);
+        tm_ldf<UH>(LA + (l1 ? C_ZG0 : C_ZG1) + uh, zg);
         tm_wait_ld();
-        float ag[16], cc[16];
+        float ag[UH], cc[UH];
 #if PDEIP_TC_PACKED
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
+        for (int i = 0; i < UH / 2; ++i) {
           const float2 g2 = __fmul2_rn(unp2(s1p, i), pr(zg, i));
           st2(ag, i, g2);
           st2(cc, i, __fadd2_rn(pr(a2, i), g2));
         }
 #else
 #pragma unroll
-        for (int i = 0; i < 16; ++i) {
+        for (int i = 0; i < UH; ++i) {
           ag[i] = unp(s1p, i) * zg[i];
           cc[i] = a2[i] + ag[i];
         }
 #endif
 #pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          put_op<kTS>(At, (AC_A1 + 2 * half + c) * 128, LOP + 4 * (2 * half + c), ag + 8 * c);
-          put_chunk(At, (AC_C + 2 * half + c) * 128, cc + 8 * c);
+        for (int c = 0; c < HC; ++c) {
+          put_op<kTS>(At, (AC_A1 + HC * part + c) * 128, LOP + 4 * (HC * part + c), ag + 8 * c);
+          put_chunk(At, (AC_C + HC * part + c) * 128, cc + 8 * c);
         }
-        TC_PROBE(l1 ? 16 : 17, u16, cc, 16);
+        TC_PROBE(l1 ? 16 : 17, uh, cc, UH);
       } else if constexpr (ph == 9) {
         // E9: s0 = s0p + 8 ug^;  db2 += s0
-        float ug[24], s0[24];
-        uint32_t spp[12];
-        tm_ldp<24>(LA + C_S0P + 12 * half, spp);
+        float ug[UO], s0[UO];
+        uint32_t spp[UO / 2];
+        oc.ldp(LA + C_S0P, spp);
+        if constexpr (kDbTmem) db2_ld(db2);
         tm_wait_ld();
         if constexpr (kEarlyLoads) wait_gemm();
-        tm_ldf<24>(LA + C_UG + u24, ug);
+        oc.ldf(LA + C_UG, ug);
         tm_wait_ld();
 #if PDEIP_TC_PACKED
 #pragma unroll
-        for (int i = 0; i < 12; ++i) {
+        for (int i = 0; i < UO / 2; ++i) {
           const float2 v = __ffma2_rn(bc2(8.f), pr(ug, i), unp2(spp, i));
           st2(s0, i, v);
           st2(db2, i, __fadd2_rn(pr(db2, i), v));
         }
 #else
 #pragma unroll
-        for (int i = 0; i < 24; ++i) {
+        for (int i = 0; i < UO; ++i) {
           s0[i] = fmaf(8.f, ug[i], unp(spp, i));
           db2[i] += s0[i];
         }
 #endif
-#pragma unroll
-        for (int c = 0; c < 3; ++c) put_op<kTS>(Z, (ZC_TA + 3 * half + c) * 128, LOP + 4 * (3 * half + c), s0 + 8 * c);
-        TC_PROBE(18, u24, s0, 24);
+        oc.template put<kTS>(Z, ZC_TA, LOP, s0);
+        if constexpr (kDbTmem) db2_st(db2);
+        TC_PROBE_OUT(18, s0);
       } else {
         // E10: zbar0' = s1_2 ab_2 + pz2 - 2 t2 aa^2 c_2;  db1       E11: zbar0'' likewise with hidden layer 1;  db0
         constexpr bool l2 = ph == 10;
@@ -1385,11 +1565,11 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         // blocking load)
 #if PDEIP_TC_L2_PREFETCH
         if constexpr (l2) {
-          if constexpr (kPipeFlow) {  // the first two items of the next tile (16 registers: x at d = 32, x and v at d = 16;
-                                      // L2 prefetch issued in E4) are read here and land behind this phase; the rest is read
-                                      // behind its hand-off, see below (measured: more than 16 registers here costs more
-                                      // in E10 than the hidden latency gives back)
-            if (tile + tile_stride < n_tiles) load_inputs(s, tile + tile_stride, 0, 2);
+          if constexpr (kPipeFlow) {  // the x and v items of the next tile (16 registers at d = 32, 8 at d = 16; L2
+                                      // prefetch issued in E4) are read here and land behind this phase (measured with 8
+                                      // epilogue warps: more than 16 registers here costs more in E10 than the hidden
+                                      // latency gives back); its stored gt is read in its own E5
+            if (tile + tile_stride < n_tiles) load_inputs(s, tile + tile_stride, 3);
           } else if (!use_stage) {
             prefetch_inputs(tile + tile_stride);
           }
@@ -1398,24 +1578,25 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         if constexpr (l2) load_inputs(s, tile + tile_stride);
 #endif
         const uint8_t* At = l2 ? A2 : A1;
-        float ab[16], aa[16], t[16], cc[16];
-        uint32_t s1p[8], pzp[8];
-        tm_ldp<16>(LA + (l2 ? C_S1P2 : C_S1P1) + 8 * half, s1p);
-        tm_ldp<16>(LA + (l2 ? C_PZ2 : C_PZ1) + 8 * half, pzp);
+        float ab[UH], aa[UH], t[UH], cc[UH];
+        uint32_t s1p[UH / 2], pzp[UH / 2];
+        tm_ldp<UH>(LA + (l2 ? C_S1P2 : C_S1P1) + UH / 2 * part, s1p);
+        tm_ldp<UH>(LA + (l2 ? C_PZ2 : C_PZ1) + UH / 2 * part, pzp);
 #pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          load_chunk(At, (AC_T + 2 * half + c) * 128, t + 8 * c);
-          load_chunk(At, (AC_C + 2 * half + c) * 128, cc + 8 * c);
+        for (int c = 0; c < HC; ++c) {
+          load_chunk(At, (AC_T + HC * part + c) * 128, t + 8 * c);
+          load_chunk(At, (AC_C + HC * part + c) * 128, cc + 8 * c);
         }
+        if constexpr (kDbTmem) db_ld(l2 ? cdb1 : cdb0, l2 ? db1 : db0);
         tm_wait_ld();
         if constexpr (kEarlyLoads) wait_gemm();
-        tm_ldf<16>(LA + (l2 ? C_AB2 : C_AB1) + u16, ab);
-        tm_ldf<16>(LA + (l2 ? C_AA2R : C_AA1R) + u16, aa);
+        tm_ldf<UH>(LA + (l2 ? C_AB2 : C_AB1) + uh, ab);
+        tm_ldf<UH>(LA + (l2 ? C_AA2R : C_AA1R) + uh, aa);
         tm_wait_ld();
-        float zb[16];
+        float zb[UH];
 #if PDEIP_TC_PACKED
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
+        for (int i = 0; i < UH / 2; ++i) {
           const float2 m0 = __ffma2_rn(unp2(s1p, i), pr(ab, i), unp2(pzp, i));
           const float2 ta = __fmul2_rn(__fmul2_rn(pr(t, i), bc2(-2.f)), pr(aa, i));
           const float2 v = __ffma2_rn(ta, pr(cc, i), m0);
@@ -1425,7 +1606,7 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         }
 #else
 #pragma unroll
-        for (int i = 0; i < 16; ++i) {
+        for (int i = 0; i < UH; ++i) {
           const float m0 = fmaf(unp(s1p, i), ab[i], unp(pzp, i));
           zb[i] = fmaf(-2.f * t[i] * aa[i], cc[i], m0);
           if (l2) db1[i] += zb[i];
@@ -1433,15 +1614,16 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         }
 #endif
 #pragma unroll
-        for (int c = 0; c < 2; ++c)  // zbar0' is an A operand of P10; zbar0'' (E11) only feeds the dW0 chain
-          put_op<(kTS && l2)>(Z, ((l2 ? ZC_TB : ZC_TA) + 2 * half + c) * 128, LOP + 4 * (2 * half + c), zb + 8 * c);
-        TC_PROBE(l2 ? 19 : 20, u16, zb, 16);
+        for (int c = 0; c < HC; ++c)  // zbar0' is an A operand of P10; zbar0'' (E11) only feeds the dW0 chain
+          put_op<(kTS && l2)>(Z, ((l2 ? ZC_TB : ZC_TA) + HC * part + c) * 128, LOP + 4 * (HC * part + c), zb + 8 * c);
+        if constexpr (kDbTmem) db_st(l2 ? cdb1 : cdb0, l2 ? db1 : db0);
+        TC_PROBE(l2 ? 19 : 20, uh, zb, UH);
       }
       if constexpr (!(kGram && ph == 6)) {  // kGram: no hand-off after E6, E7 follows immediately (zg^_0 came out of P5)
         if constexpr (kTS) tm_wait_st();  // the A-operand columns are complete before the hand-off
         TC_TRACE(7);
         if constexpr (kTwoStage && (ph == 3 || ph == 4 || ph == 5 || ph == 7 || ph == 9 || ph == 10 || ph == 11)) {
-          epi_arrive<false>(s);  // layer GEMMs (A from TMEM, B = weights): go
+          epi_arrive<NS, false>(s);  // layer GEMMs (A from TMEM, B = weights): go
           fence_async_smem();    // the bands this phase wrote -> async proxy, for the dW chains behind the second barrier
           asm volatile("bar.arrive %0, %1;" ::"r"(4 + (int)tsb), "n"(kThreads) : "memory");
           tsb ^= 1u;
@@ -1458,22 +1640,17 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
         // memory, and the bands written by E0, E1, E2, E8 are first read by dW chains issued behind LATER hand-offs
         // (P3 / P4 / P5 / P9 ...), whose fences (same thread, later in program order) cover these writes too.
         constexpr bool kNeedProxyFence = !(kTS && (ph == 0 || ph == 1 || ph == 2 || ph == 8));
-        epi_arrive<kNeedProxyFence>(s);
+        epi_arrive<NS, kNeedProxyFence>(s);
 #endif
         }
         TC_TRACE(2);
       }
       if constexpr (kPipeFlow && ph == 10) {  // E0 of the NEXT tile, while P10 executes (its TMEM stores and shared-memory
                                           // writes are ordered before P0 by the wait::st / proxy fence of E11's hand-off)
-        // The inputs were pulled into L2 one tile ago; the loads are issued HERE and not at the start of E10: with the
-        // 48 input registers live across E10 the compiler parks them in local memory, and the store behind each load
-        // sits out the full memory latency in front of the wait for P9 (phase trace: +1.8 k cycles per tile at d = 32).
+        // (its x and v items were read at the start of E10)
         const int64_t tn = tile + tile_stride;
         const int64_t pn = (FPM ? (int64_t)((uint32_t)tn / fpd) : tn) * 128 + row;
-        if (tn < n_tiles) {
-          load_inputs(s, tn, 2, 64);
-          emit_x(xin0, pn < a.n_points, sm + (xb ? 0u : S::O_X2) + S::O_X + offX);
-        }
+        if (tn < n_tiles) emit_x(xin0, pn < a.n_points, sm + (xb ? 0u : S::O_X2) + S::O_X + offX);
       }
     };
 #define PDEIP_TC_PHASE(PH)                       \
@@ -1500,45 +1677,59 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
     asm volatile("bar.sync 3, %0;" ::"n"(kEpiThreads) : "memory");
 
     // ---- write-out: this CTA's partial (one writer per index, fixed order -> bit-reproducible) ------------------
-    float* part = a.ws + (int64_t)blockIdx.x * a.pstride;
-    float* red = reinterpret_cast<float*>(sm);  // [4 quadrants][128] bias sums + [8 warps][8] loss sums
+    float* wsp = a.ws + (int64_t)blockIdx.x * a.pstride;
+    float* red = reinterpret_cast<float*>(sm);  // [4 quadrants][128] bias sums + [epilogue warps][8] loss sums
+    static_assert((512 + 8 * Team<NS>::kEpiWarps) * 4 <= S::O_BIAS, "write-out scratch inside the operand tiles");
     const float wt = a.weight;
     if (ok && q < 2) {  // M = 64 dW blocks: input unit i = 16 q + lane sits in TMEM lane 32 q + lane, lane < 16
       const uint32_t LQ = TB + ((uint32_t)(q * 32) << 16);
       const int iu = 16 * q + lane;
-      float w2[24], w1[16], w0[16];
-      tm_ldf<24>(LQ + C_DW2 + u24, w2);
-      tm_ldf<16>(LQ + C_DW1 + u16, w1);
-      tm_ldf<16>(LQ + C_DW0 + u16, w0);
+      float w2[UO], w1[UH], w0[UH];
+      oc.ldf(LQ + C_DW2, w2);
+      tm_ldf<UH>(LQ + C_DW1 + uh, w1);
+      tm_ldf<UH>(LQ + C_DW0 + uh, w0);
       tm_wait_ld();
       if (lane < 16) {
 #pragma unroll
-        for (int i = 0; i < 24; ++i)
-          if (u24 + i < kOut) part[sh.w_off(2) + iu * kOut + u24 + i] += wt * w2[i];
+        for (int i = 0; i < UO; ++i)
+          if (oc.unit(i) < kOut) wsp[sh.w_off(2) + iu * kOut + oc.unit(i)] += wt * w2[i];
 #pragma unroll
-        for (int i = 0; i < 16; ++i) part[sh.w_off(1) + iu * H + u16 + i] += wt * w1[i];
+        for (int i = 0; i < UH; ++i) wsp[sh.w_off(1) + iu * H + uh + i] += wt * w1[i];
         if (iu < d) {
 #pragma unroll
-          for (int i = 0; i < 16; ++i) part[sh.w_off(0) + iu * H + u16 + i] += wt * w0[i];
+          for (int i = 0; i < UH; ++i) wsp[sh.w_off(0) + iu * H + uh + i] += wt * w0[i];
         }
       }
     }
     // bias gradients: sum over the 32 rows of the warp, then over the 4 quadrants through shared memory
     // red layout: [q][0..31] db0, [32..63] db1, [64..111] db2
+    if constexpr (kDbTmem) {
+      db_ld(cdb0, db0);
+      db_ld(cdb1, db1);
+      db2_ld(db2);
+      tm_wait_ld();
+    }
 #pragma unroll
-    for (int i = 0; i < 16; ++i) {
+    for (int i = 0; i < UH; ++i) {
       const float r0 = warp_sum(db0[i]), r1 = warp_sum(db1[i]);
       if (lane == 0) {
-        red[q * 128 + u16 + i] = r0;
-        red[q * 128 + 32 + u16 + i] = r1;
+        red[q * 128 + uh + i] = r0;
+        red[q * 128 + 32 + uh + i] = r1;
       }
     }
 #pragma unroll
-    for (int i = 0; i < 24; ++i) {
+    for (int i = 0; i < UO; ++i) {
       const float r2 = warp_sum(db2[i]);
-      if (lane == 0) red[q * 128 + 64 + u24 + i] = r2;
+      if (lane == 0) red[q * 128 + 64 + oc.unit(i)] = r2;
     }
     {
+      if constexpr (kSumsSmem) {
+        sum_g2 = sums_s[0];
+        sum_gt2 = sums_s[kEpiThreads];
+        sum_gd2 = sums_s[2 * kEpiThreads];
+        sum_d1 = sums_s[3 * kEpiThreads];
+        sum_d2 = sums_s[4 * kEpiThreads];
+      }
       const float sums5[5] = {sum_g2, sum_gt2, sum_gd2, sum_d1, sum_d2};
 #pragma unroll
       for (int k = 0; k < 5; ++k) {
@@ -1550,25 +1741,25 @@ __global__ void __launch_bounds__(kLaunchThreads, 1) mlp_residual_tc_kernel(cons
     if (ok) {
       if (tid < 112) {
         const float v = (red[tid] + red[128 + tid]) + (red[256 + tid] + red[384 + tid]);
-        if (tid < 32) part[sh.b_off(0) + tid] += wt * v;
-        else if (tid < 64) part[sh.b_off(1) + tid - 32] += wt * v;
-        else if (tid - 64 < kOut) part[sh.b_off(2) + tid - 64] += wt * v;
+        if (tid < 32) wsp[sh.b_off(0) + tid] += wt * v;
+        else if (tid < 64) wsp[sh.b_off(1) + tid - 32] += wt * v;
+        else if (tid - 64 < kOut) wsp[sh.b_off(2) + tid - 64] += wt * v;
       }
       if (tid == 128) {
         float t5[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
-        for (int w = 0; w < kEpiThreads / 32; ++w)
+        for (int w = 0; w < Team<NS>::kEpiWarps; ++w)
           for (int k = 0; k < 5; ++k) t5[k] += red[512 + w * 8 + k];
         const float g2 = wt * t5[0], gt2 = wt * t5[1], gd2 = wt * t5[2], D1 = wt * t5[3], D2 = wt * t5[4];
         if constexpr (BND) {  // residual_mlp.cu, KFP_BOUNDARY: sum coef grad V . v
-          part[P + PDEIP_SUM_BOUNDARY] += a.coef * D1;
-          part[P + PDEIP_SUM_LOSS] += a.coef * D1;
+          wsp[P + PDEIP_SUM_BOUNDARY] += a.coef * D1;
+          wsp[P + PDEIP_SUM_LOSS] += a.coef * D1;
         } else {
-          part[P + PDEIP_SUM_G2] += g2;
-          part[P + PDEIP_SUM_GTRUE2] += gt2;
-          part[P + PDEIP_SUM_GT] += gd2;
-          if (!FPM) part[P + PDEIP_SUM_D1] += D1;  // FP rows: D_{e_i} V is not a loss term (fokker_planck.py:50-51)
-          part[P + PDEIP_SUM_D2] += D2;
-          part[P + PDEIP_SUM_LOSS] += g2 + gt2 - 2.f * D2 + 2.f * gamma * D1;
+          wsp[P + PDEIP_SUM_G2] += g2;
+          wsp[P + PDEIP_SUM_GTRUE2] += gt2;
+          wsp[P + PDEIP_SUM_GT] += gd2;
+          if (!FPM) wsp[P + PDEIP_SUM_D1] += D1;  // FP rows: D_{e_i} V is not a loss term (fokker_planck.py:50-51)
+          wsp[P + PDEIP_SUM_D2] += D2;
+          wsp[P + PDEIP_SUM_LOSS] += g2 + gt2 - 2.f * D2 + 2.f * gamma * D1;
         }
       }
     }
@@ -1602,7 +1793,7 @@ static int launch_tc(const ResidualArgs& a, int* status, cudaStream_t st) {
   PDEIP_REQUIRE(true_grad_floats(a.tg, a.d) * sizeof(float) <= S::TP_BYTES, PDEIP_ERR_UNSUPPORTED,
                 "tensor path: true-gradient parameters exceed %u bytes", (unsigned)S::TP_BYTES);
   PDEIP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL));
-  kern<<<residual_grid(), tc::kLaunchThreads, S::TOTAL, st>>>(a, status);
+  kern<<<residual_grid(), tc::Team<NS>::kLaunchThreads, S::TOTAL, st>>>(a, status);
   PDEIP_LAUNCH_OK();
   return PDEIP_OK;
 }
