@@ -155,6 +155,44 @@ int pdeip_kl_integrate_model(const float* z0, float* z_last, float* traj, float*
                              int schedule, int state_layout, int traj_layout,
                              int emit_every, int emit_offset, int emit_drift, int path, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * K1-OD  overdamped Langevin integrator: dX = -grad U(X) dt + sqrt(2) dW (the Fokker-Planck instance,
+ * example_problems/fokker_planck_example.py), Euler-Maruyama with S steps of size dt:
+ *   x_{s+1} = x_s - dt grad U(x_s) + sqrt(2 dt) xi_s,   s = 0..S-1   (the sqrt(2) is fixed, as in K1)
+ * Sample s is the state after step s; x_last is sample S-1.  No tau0, no reference schedule.
+ * x0, x_last: [N][d] (state_layout AOS) or [d][N] (SOA).  noise: NULL -> Philox4x32-10 keyed by (seed, particle_offset
+ * + n, step_offset + s), i.e. draw s of pdeip_philox_normals(n, S, d, seed, particle_offset, step_offset); else injected
+ * normals [N][S][d].  traj: NULL for terminal-only, else sample s is emitted iff s % emit_every == emit_offset, in the
+ * four K1 trajectory layouts with C = d components per sample, or C = 2d with emit_drift: [x, grad U(x)] (the drift
+ * step s+1 evaluates anyway; the last sample takes one extra evaluation).  A PDEIP_TRAJ_BLOCK128 trajectory is directly
+ * a PDEIP_LAYOUT_BLOCK128 FP point set, with PDEIP_DRIFT_IN_POINTS when the drift is emitted.
+ * Drifts: PDEIP_DRIFT_NONE / _LINEAR / _GMM / _MEANFIELD, fp32 on the CUDA cores on both paths (the GMM drift has no
+ * overdamped tcgen05 kernel).  PDEIP_DRIFT_MEANFIELD_TABLE encodes the underdamped mean recursion and is rejected
+ * (PDEIP_ERR_UNSUPPORTED).  Rejected before any CUDA call, with a pdeip_last_error message: unknown drift kind, path or
+ * layout, NULL x0 or drift_params, n_steps < 1, bad emit_every / emit_offset (PDEIP_ERR_INVALID_ARG), BLOCK128 with
+ * n % 128 != 0 (PDEIP_ERR_INVALID_ARG), d outside [1, 32] (PDEIP_ERR_UNSUPPORTED).
+ * ------------------------------------------------------------------------------------------- */
+int pdeip_overdamped_integrate(const float* x0, float* x_last, float* traj, int64_t n_particles, int d, int n_steps,
+                               float dt, int drift_kind, const float* drift_params, int n_gaussian, float sigma,
+                               const float* noise, uint64_t seed, uint64_t particle_offset, uint32_t step_offset,
+                               int state_layout, int traj_layout, int emit_every, int emit_offset, int emit_drift,
+                               int path, void* stream);
+
+/* K1-OD with grad U = grad V_theta of a hypothesis model, with the envelope and rejections of pdeip_kl_integrate_model:
+ *   PDEIP_MODEL_MLP       hidden == 32, 1 <= layers <= 8, d <= 32, fp32 on the CUDA cores.  PDEIP_PATH_TENSOR with
+ *                         layers == 2, d = 8, 16 or 32, Philox noise, AOS state, emit_every 1 and either traj == NULL
+ *                         (terminal state only, n arbitrary) or a PDEIP_TRAJ_BLOCK128 / PDEIP_TRAJ_TIME_SOA trajectory
+ *                         with emit_drift runs the six GEMMs of a step on tcgen05 (K1-MT, bf16 hi + lo split operands);
+ *                         every other call takes the fp32 kernel, bit-identical to PDEIP_PATH_FP32
+ *                         (PDEIP_NO_TC_INTEGRATOR=1 forces it);
+ *   PDEIP_MODEL_GMM       exactly pdeip_overdamped_integrate(PDEIP_DRIFT_GMM, params, n_gaussian, 1.0f, ...);
+ *   PDEIP_MODEL_QUADRATIC grad V = (K + K^T) y + b, fp32 on both paths. */
+int pdeip_overdamped_integrate_model(const float* x0, float* x_last, float* traj, int64_t n_particles, int d,
+                                     int n_steps, float dt, int model_kind, const float* params, int hidden, int layers,
+                                     int n_gaussian, const float* noise, uint64_t seed, uint64_t particle_offset,
+                                     uint32_t step_offset, int state_layout, int traj_layout, int emit_every,
+                                     int emit_offset, int emit_drift, int path, void* stream);
+
 /* Mean-field drift (interacting system, README.md:54-62): the ensemble mean on the common time grid obeys
  *   pbar' = (1 - gamma dt) pbar + sqrt(2 dt) xibar_s,  qbar' = qbar + dt pbar'   (the interaction cancels in the mean),
  * xibar_s = mean over ALL particles of the step-s Philox normals.  noise_sums accumulates (atomically, caller zeroes)

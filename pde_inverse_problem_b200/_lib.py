@@ -52,6 +52,10 @@ SIGNATURES: Dict[str, tuple] = {
                                      _i, _i, _i, _i, _i, _i, _i, _p]),
     "pdeip_kl_integrate_model": (_i, [_p, _p, _p, _p, _l, _i, _i, _f, _f, _i, _p, _i, _i, _i, _p, _p, _u64, _u64, _u32,
                                       _i, _i, _i, _i, _i, _i, _i, _p]),
+    "pdeip_overdamped_integrate": (_i, [_p, _p, _p, _l, _i, _i, _f, _i, _p, _i, _f, _p, _u64, _u64, _u32, _i, _i, _i,
+                                        _i, _i, _i, _p]),
+    "pdeip_overdamped_integrate_model": (_i, [_p, _p, _p, _l, _i, _i, _f, _i, _p, _i, _i, _i, _p, _u64, _u64, _u32,
+                                              _i, _i, _i, _i, _i, _i, _p]),
     "pdeip_philox_normals": (_i, [_p, _l, _i, _i, _u64, _u64, _u32, _p]),
     "pdeip_philox_uniforms": (_i, [_p, _l, _u64, _u64, _p]),
     "pdeip_philox_raw": (_i, [_p, _p, _p, _l, _p]),

@@ -91,12 +91,40 @@ __device__ __forceinline__ void emit_drift_vals(float* __restrict__ base, int la
   }
 }
 
+// v[0, d) -> components [col0, col0 + d) of sample s_e (row width C) in any trajectory layout (overdamped K1-OD)
+template <int DP>
+__device__ __forceinline__ void emit_cols(float* __restrict__ base, int layout, int64_t n, int64_t n_total, int d,
+                                          int C, int col0, int s_e, int s_emit, const float (&v)[DP]) {
+  if (layout == PDEIP_TRAJ_BLOCK128) {
+    float* o = base + (((int64_t)s_e * (n_total >> 7) + (n >> 7)) * C + col0) * 128 + (n & 127);
+#pragma unroll
+    for (int i = 0; i < DP; ++i)
+      if (i < d) __stcs(o + i * 128, v[i]);
+    return;
+  }
+  if (layout == PDEIP_TRAJ_TIME_SOA) {
+    const int64_t plane = (int64_t)s_emit * n_total;
+    float* o = base + (int64_t)col0 * plane + (int64_t)s_e * n_total + n;
+#pragma unroll
+    for (int i = 0; i < DP; ++i)
+      if (i < d) __stcs(o + (int64_t)i * plane, v[i]);
+    return;
+  }
+  float* o = (layout == PDEIP_TRAJ_PARTICLE_MAJOR) ? base + (n * s_emit + s_e) * C + col0
+                                                    : base + ((int64_t)s_e * n_total + n) * C + col0;
+#pragma unroll
+  for (int i = 0; i < DP; ++i)
+    if (i < d) __stcs(o + i, v[i]);
+}
+
 // drift kinds of the hypothesis models (pdeip_kl_integrate_model), internal to this file
 constexpr int kDriftAffine = 100;  // quadratic model: grad V = (K + K^T) y + b, params = [K (d*d), b (d)]
 constexpr int kDriftMlp = 101;     // MLP model: grad V_theta, params = the flat MLP buffer (hidden width 32)
 
-// LHMAX: hidden layers the per-thread MLP state is sized for (kDriftMlp only)
-template <int DP, int DRIFT, int LHMAX = 0>
+// LHMAX: hidden layers the per-thread MLP state is sized for (kDriftMlp only).
+// OD: overdamped dynamics (pdeip_overdamped_integrate*): the state is x alone, x' = x - h grad U(x) + sqrt(2h) xi, on
+// the UNIFORM schedule; an emitted sample is [x] or [x, grad U(x)].  OD = false is the kinetic K1 step.
+template <int DP, int DRIFT, int LHMAX = 0, bool OD = false>
 __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a) {
   extern __shared__ __align__(16) float smem[];
   // stage the drift parameters (zero-padded to DP) in shared memory
@@ -137,8 +165,12 @@ __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a
   float q[DP], p[DP];
 #pragma unroll
   for (int i = 0; i < DP; ++i) {
-    q[i] = (i < d) ? a.z0[elem_index(a.state_layout, n, i, a.n, 2 * d)] : 0.0f;
-    p[i] = (i < d) ? a.z0[elem_index(a.state_layout, n, d + i, a.n, 2 * d)] : 0.0f;
+    if constexpr (OD) {
+      q[i] = (i < d) ? a.z0[elem_index(a.state_layout, n, i, a.n, d)] : 0.0f;
+    } else {
+      q[i] = (i < d) ? a.z0[elem_index(a.state_layout, n, i, a.n, 2 * d)] : 0.0f;
+      p[i] = (i < d) ? a.z0[elem_index(a.state_layout, n, d + i, a.n, 2 * d)] : 0.0f;
+    }
   }
 
   const bool ref_sched = (a.schedule == PDEIP_SCHEDULE_REFERENCE);
@@ -149,7 +181,7 @@ __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a
   }
   const int total_steps = ref_sched ? a.n_steps + 1 : a.n_steps;
   const int n_draws = total_steps;
-  const int C = a.emit_drift ? 3 * d : 2 * d;  // floats per emitted sample
+  const int C = OD ? (a.emit_drift ? 2 * d : d) : (a.emit_drift ? 3 * d : 2 * d);  // floats per emitted sample
 
   for (int s = 0; s < total_steps; ++s) {
     float h = a.dt;
@@ -178,8 +210,10 @@ __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a
       for (int i = 0; i < DP; ++i) g[i] = 0.0f;
     }
     // the drift just evaluated is grad U at the state emitted as sample s-1
-    if (a.emit_drift && a.traj && s >= 1 && ((s - 1) % a.emit_every) == a.emit_offset)
-      emit_drift_vals<DP>(a.traj, a.traj_layout, n, a.n, d, C, (s - 1) / a.emit_every, a.s_emit, g);
+    if (a.emit_drift && a.traj && s >= 1 && ((s - 1) % a.emit_every) == a.emit_offset) {
+      if constexpr (OD) emit_cols<DP>(a.traj, a.traj_layout, n, a.n, d, C, d, (s - 1) / a.emit_every, a.s_emit, g);
+      else emit_drift_vals<DP>(a.traj, a.traj_layout, n, a.n, d, C, (s - 1) / a.emit_every, a.s_emit, g);
+    }
     // noise
     float xi[DP];
     if (a.noise) {
@@ -200,15 +234,20 @@ __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a
     const float sq = sqrtf(h) * 1.41421356237309515f;
 #pragma unroll
     for (int i = 0; i < DP; ++i) {
-      const float pn = p[i] - h * g[i] + sq * xi[i] - a.gamma * p[i] * h;
-      p[i] = pn;
-      q[i] = q[i] + h * pn;
+      if constexpr (OD) {  // x' = x - h grad U(x) + sqrt(h) sqrt(2) xi
+        q[i] = q[i] - h * g[i] + sq * xi[i];
+      } else {
+        const float pn = p[i] - h * g[i] + sq * xi[i] - a.gamma * p[i] * h;
+        p[i] = pn;
+        q[i] = q[i] + h * pn;
+      }
     }
     // emission: REFERENCE schedule emits samples 0..S-1 (the last step only feeds z_last);
     // UNIFORM schedule emits every state.
     const bool is_sample = ref_sched ? (s < a.n_steps) : true;
     if (a.traj && is_sample && (s % a.emit_every) == a.emit_offset) {
-      emit_state<DP>(a.traj, a.traj_layout, n, a.n, d, C, s / a.emit_every, a.s_emit, q, p);
+      if constexpr (OD) emit_cols<DP>(a.traj, a.traj_layout, n, a.n, d, C, 0, s / a.emit_every, a.s_emit, q);
+      else emit_state<DP>(a.traj, a.traj_layout, n, a.n, d, C, s / a.emit_every, a.s_emit, q, p);
     }
   }
   if (a.emit_drift && a.traj && !ref_sched && ((total_steps - 1) % a.emit_every) == a.emit_offset) {
@@ -226,14 +265,19 @@ __global__ void __launch_bounds__(128) kl_integrate_kernel(const IntegrateArgs a
 #pragma unroll
       for (int i = 0; i < DP; ++i) g[i] = 0.0f;
     }
-    emit_drift_vals<DP>(a.traj, a.traj_layout, n, a.n, d, C, (total_steps - 1) / a.emit_every, a.s_emit, g);
+    if constexpr (OD) emit_cols<DP>(a.traj, a.traj_layout, n, a.n, d, C, d, (total_steps - 1) / a.emit_every, a.s_emit, g);
+    else emit_drift_vals<DP>(a.traj, a.traj_layout, n, a.n, d, C, (total_steps - 1) / a.emit_every, a.s_emit, g);
   }
   if (a.z_last) {
 #pragma unroll
     for (int i = 0; i < DP; ++i)
       if (i < d) {
-        a.z_last[elem_index(a.state_layout, n, i, a.n, 2 * d)] = q[i];
-        a.z_last[elem_index(a.state_layout, n, d + i, a.n, 2 * d)] = p[i];
+        if constexpr (OD) {
+          a.z_last[elem_index(a.state_layout, n, i, a.n, d)] = q[i];
+        } else {
+          a.z_last[elem_index(a.state_layout, n, i, a.n, 2 * d)] = q[i];
+          a.z_last[elem_index(a.state_layout, n, d + i, a.n, 2 * d)] = p[i];
+        }
       }
   }
   if (a.tau && ref_sched) {
@@ -546,6 +590,49 @@ static int launch_integrate_model(const IntegrateArgs& a, int model_kind, int pa
   return PDEIP_OK;
 }
 
+// K1-OD: the overdamped step on the generic kernel, every analytic drift and configuration (the entry point has
+// rejected PDEIP_DRIFT_MEANFIELD_TABLE and unknown kinds)
+template <int DP>
+static int launch_overdamped(const IntegrateArgs& a, int drift_kind, cudaStream_t st) {
+  const unsigned grid = (unsigned)((a.n + 127) / 128);
+  switch (drift_kind) {
+    case PDEIP_DRIFT_NONE:
+      kl_integrate_kernel<DP, PDEIP_DRIFT_NONE, 0, true><<<grid, 128, 0, st>>>(a);
+      break;
+    case PDEIP_DRIFT_LINEAR:
+      kl_integrate_kernel<DP, PDEIP_DRIFT_LINEAR, 0, true><<<grid, 128, sizeof(float) * DP * DP, st>>>(a);
+      break;
+    case PDEIP_DRIFT_MEANFIELD:
+      kl_integrate_kernel<DP, PDEIP_DRIFT_MEANFIELD, 0, true><<<grid, 128, sizeof(float) * (DP * DP + DP), st>>>(a);
+      break;
+    default: {  // PDEIP_DRIFT_GMM
+      const size_t smem = sizeof(float) * (size_t)a.n_gaussian * DP;
+      PDEIP_REQUIRE(smem <= 48 * 1024, PDEIP_ERR_UNSUPPORTED, "GMM centres exceed 48 KB of shared memory");
+      kl_integrate_kernel<DP, PDEIP_DRIFT_GMM, 0, true><<<grid, 128, smem, st>>>(a);
+    }
+  }
+  PDEIP_LAUNCH_OK();
+  return PDEIP_OK;
+}
+
+// K1-OD under a hypothesis model's potential; under PDEIP_PATH_TENSOR the MLP drift of the tcgen05 kernel's envelope
+template <int DP>
+static int launch_overdamped_model(const IntegrateArgs& a, int model_kind, int path, cudaStream_t st) {
+  if (model_kind == PDEIP_MODEL_MLP && path == PDEIP_PATH_TENSOR && overdamped_mlp_tensor_ok(a))
+    return launch_overdamped_mlp_tensor(a, st);
+  const unsigned grid = (unsigned)((a.n + 127) / 128);
+  if (model_kind == PDEIP_MODEL_QUADRATIC) {
+    kl_integrate_kernel<DP, kDriftAffine, 0, true><<<grid, 128, sizeof(float) * (DP * DP + DP), st>>>(a);
+  } else {
+    const size_t smem = sizeof(float) * (size_t)MlpShape<32>{a.d, a.layers}.num_params();
+    if (a.layers <= 2) kl_integrate_kernel<DP, kDriftMlp, 2, true><<<grid, 128, smem, st>>>(a);
+    else if (a.layers <= 4) kl_integrate_kernel<DP, kDriftMlp, 4, true><<<grid, 128, smem, st>>>(a);
+    else kl_integrate_kernel<DP, kDriftMlp, 8, true><<<grid, 128, smem, st>>>(a);
+  }
+  PDEIP_LAUNCH_OK();
+  return PDEIP_OK;
+}
+
 // ------------------------------------------------------------------------------------------
 // noise dumps (what the integrator draws in Philox mode) and the Gaussian initial ensemble
 // ------------------------------------------------------------------------------------------
@@ -789,6 +876,85 @@ extern "C" int pdeip_kl_integrate_model(const float* z0, float* z_last, float* t
   if (d <= 8) return launch_integrate_model<8>(a, model_kind, path, st);
   if (d <= 16) return launch_integrate_model<16>(a, model_kind, path, st);
   return launch_integrate_model<32>(a, model_kind, path, st);
+}
+
+// the arguments of the overdamped entry points: those of K1 on the UNIFORM schedule with no friction, tau or tau0
+static int overdamped_args(IntegrateArgs& a, const float* x0, float* x_last, float* traj, int64_t n_particles, int d,
+                           int n_steps, float dt, const float* noise, uint64_t seed, uint64_t particle_offset,
+                           uint32_t step_offset, int state_layout, int traj_layout, int emit_every, int emit_offset,
+                           int emit_drift, int path) {
+  PDEIP_REQUIRE(x0 != nullptr, PDEIP_ERR_INVALID_ARG, "x0 is NULL");
+  return integrate_args(a, x0, x_last, traj, nullptr, n_particles, d, n_steps, dt, 0.0f, noise, nullptr, seed,
+                        particle_offset, step_offset, PDEIP_SCHEDULE_UNIFORM, state_layout, traj_layout, emit_every,
+                        emit_offset, emit_drift, path);
+}
+
+extern "C" int pdeip_overdamped_integrate(const float* x0, float* x_last, float* traj, int64_t n_particles, int d,
+                                          int n_steps, float dt, int drift_kind, const float* drift_params,
+                                          int n_gaussian, float sigma, const float* noise, uint64_t seed,
+                                          uint64_t particle_offset, uint32_t step_offset, int state_layout,
+                                          int traj_layout, int emit_every, int emit_offset, int emit_drift, int path,
+                                          void* stream) {
+  PDEIP_REQUIRE(drift_kind != PDEIP_DRIFT_MEANFIELD_TABLE, PDEIP_ERR_UNSUPPORTED,
+                "PDEIP_DRIFT_MEANFIELD_TABLE encodes the underdamped mean recursion; the overdamped step does not take it");
+  PDEIP_REQUIRE(drift_kind == PDEIP_DRIFT_NONE || drift_kind == PDEIP_DRIFT_LINEAR || drift_kind == PDEIP_DRIFT_GMM ||
+                    drift_kind == PDEIP_DRIFT_MEANFIELD,
+                PDEIP_ERR_INVALID_ARG, "unknown drift kind %d", drift_kind);
+  IntegrateArgs a;
+  const int rc = overdamped_args(a, x0, x_last, traj, n_particles, d, n_steps, dt, noise, seed, particle_offset,
+                                 step_offset, state_layout, traj_layout, emit_every, emit_offset, emit_drift, path);
+  if (rc != PDEIP_OK) return rc;
+  PDEIP_REQUIRE(drift_kind == PDEIP_DRIFT_NONE || drift_params != nullptr, PDEIP_ERR_INVALID_ARG,
+                "drift_params is NULL");
+  PDEIP_REQUIRE(drift_kind != PDEIP_DRIFT_GMM || (n_gaussian >= 1 && sigma > 0.0f), PDEIP_ERR_INVALID_ARG,
+                "GMM drift needs n_gaussian >= 1 and sigma > 0");
+  if (n_particles == 0) return PDEIP_OK;
+  a.drift_params = drift_params;
+  a.n_gaussian = n_gaussian; a.inv_sigma2 = drift_kind == PDEIP_DRIFT_GMM ? 1.0f / (sigma * sigma) : 1.0f;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (d <= 2) return launch_overdamped<2>(a, drift_kind, st);
+  if (d <= 4) return launch_overdamped<4>(a, drift_kind, st);
+  if (d <= 8) return launch_overdamped<8>(a, drift_kind, st);
+  if (d <= 16) return launch_overdamped<16>(a, drift_kind, st);
+  return launch_overdamped<32>(a, drift_kind, st);
+}
+
+extern "C" int pdeip_overdamped_integrate_model(const float* x0, float* x_last, float* traj, int64_t n_particles,
+                                                int d, int n_steps, float dt, int model_kind, const float* params,
+                                                int hidden, int layers, int n_gaussian, const float* noise,
+                                                uint64_t seed, uint64_t particle_offset, uint32_t step_offset,
+                                                int state_layout, int traj_layout, int emit_every, int emit_offset,
+                                                int emit_drift, int path, void* stream) {
+  PDEIP_REQUIRE(model_kind == PDEIP_MODEL_MLP || model_kind == PDEIP_MODEL_GMM || model_kind == PDEIP_MODEL_QUADRATIC,
+                PDEIP_ERR_INVALID_ARG, "unknown model kind %d", model_kind);
+  PDEIP_REQUIRE(params != nullptr, PDEIP_ERR_INVALID_ARG, "params is NULL");
+  PDEIP_REQUIRE(d >= 1 && d <= 32, PDEIP_ERR_UNSUPPORTED, "integrator supports 1 <= d <= 32 (got d=%d)", d);
+  if (model_kind == PDEIP_MODEL_GMM) {
+    // the parametric GMM model (learned centres, sigma = 1) is exactly the GMM drift
+    PDEIP_REQUIRE(n_gaussian >= 1, PDEIP_ERR_INVALID_ARG, "GMM model needs n_gaussian >= 1 (got %d)", n_gaussian);
+    return pdeip_overdamped_integrate(x0, x_last, traj, n_particles, d, n_steps, dt, PDEIP_DRIFT_GMM, params,
+                                      n_gaussian, 1.0f, noise, seed, particle_offset, step_offset, state_layout,
+                                      traj_layout, emit_every, emit_offset, emit_drift, path, stream);
+  }
+  if (model_kind == PDEIP_MODEL_MLP) {
+    PDEIP_REQUIRE(hidden == 32, PDEIP_ERR_UNSUPPORTED,
+                  "MLP drift is built for hidden_dim == 32 (pad smaller widths with zeros); got %d", hidden);
+    PDEIP_REQUIRE(layers >= 1 && layers <= 8, PDEIP_ERR_UNSUPPORTED, "MLP drift supports 1 <= layers <= 8 (got %d)",
+                  layers);
+  }
+  IntegrateArgs a;
+  const int rc = overdamped_args(a, x0, x_last, traj, n_particles, d, n_steps, dt, noise, seed, particle_offset,
+                                 step_offset, state_layout, traj_layout, emit_every, emit_offset, emit_drift, path);
+  if (rc != PDEIP_OK) return rc;
+  if (n_particles == 0) return PDEIP_OK;
+  a.drift_params = params;
+  a.layers = model_kind == PDEIP_MODEL_MLP ? layers : 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (d <= 2) return launch_overdamped_model<2>(a, model_kind, path, st);
+  if (d <= 4) return launch_overdamped_model<4>(a, model_kind, path, st);
+  if (d <= 8) return launch_overdamped_model<8>(a, model_kind, path, st);
+  if (d <= 16) return launch_overdamped_model<16>(a, model_kind, path, st);
+  return launch_overdamped_model<32>(a, model_kind, path, st);
 }
 
 extern "C" int pdeip_kl_integrate(const float* z0, float* z_last, float* traj, float* tau,

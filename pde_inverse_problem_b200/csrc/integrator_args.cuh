@@ -44,5 +44,8 @@ int launch_integrate_tensor(const IntegrateArgs& a, cudaStream_t st);
 // integrator_mlp_tc.cu: MLP (32 x 2) drift on the tensor cores (PDEIP_PATH_TENSOR of pdeip_kl_integrate_model)
 bool integrate_mlp_tensor_ok(const IntegrateArgs& a);
 int launch_integrate_mlp_tensor(const IntegrateArgs& a, cudaStream_t st);
+// ... and its overdamped variant (PDEIP_PATH_TENSOR of pdeip_overdamped_integrate_model)
+bool overdamped_mlp_tensor_ok(const IntegrateArgs& a);
+int launch_overdamped_mlp_tensor(const IntegrateArgs& a, cudaStream_t st);
 
 }  // namespace pdeip

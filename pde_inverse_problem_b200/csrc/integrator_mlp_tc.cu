@@ -17,6 +17,11 @@
 // are fp32.  The step's Philox normals are drawn while F0 is in flight.  Bounded mbarrier waits set status word 1 (the
 // integrator word) on a timeout, as kl_integrate_tc_kernel does.  Same Philox stream, tau0, step schedule and outputs
 // as the fp32 kernel of pdeip_kl_integrate_model.
+//
+// OD = true is the overdamped variant (PDEIP_PATH_TENSOR of pdeip_overdamped_integrate_model): the state per thread is
+// x alone, S steps x' = x - dt grad V_theta(x) + sqrt(2 dt) xi with no tau0; x + sqrt(2 dt) xi is formed while F0 runs
+// and B0's epilogue subtracts dt grad V_theta and emits [x, grad V_theta].  A trajectory run makes one extra drift
+// evaluation (GEMM chain without an update) for the last sample's drift.  Same weight tiles, TMEM map and hand-offs.
 #include "common.cuh"
 #include "integrator_args.cuh"
 #include "mlp_thread.cuh"
@@ -102,7 +107,7 @@ __device__ __forceinline__ void stage_weight(uint8_t* hi_t, uint8_t* lo_t, uint3
 }
 
 // TRAJ: 0 = terminal state only, 1 = PDEIP_TRAJ_BLOCK128, 2 = PDEIP_TRAJ_TIME_SOA (both with grad V_theta)
-template <int DP, int TRAJ, int MINB>
+template <int DP, int TRAJ, int MINB, bool OD = false>
 __global__ void __launch_bounds__(128, MINB) kl_integrate_mlp_tc_kernel(const IntegrateArgs a, int* status) {
   using S = Cfg<DP>;
   constexpr int DK = S::DK;
@@ -156,7 +161,14 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_mlp_tc_kernel(const In
   const int64_t n = n_raw < a.n ? n_raw : a.n - 1;
   const uint64_t pid = a.particle_offset + (uint64_t)n;
   float q[DP], p[DP];
-  {
+  if constexpr (OD) {
+    const float4* z4 = reinterpret_cast<const float4*>(a.z0 + n * DP);
+#pragma unroll
+    for (int i4 = 0; i4 < DP / 4; ++i4) {
+      const float4 tq = z4[i4];
+      q[4 * i4] = tq.x; q[4 * i4 + 1] = tq.y; q[4 * i4 + 2] = tq.z; q[4 * i4 + 3] = tq.w;
+    }
+  } else {
     const float4* z4 = reinterpret_cast<const float4*>(a.z0 + n * (2 * DP));
 #pragma unroll
     for (int i4 = 0; i4 < DP / 4; ++i4) {
@@ -165,12 +177,15 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_mlp_tc_kernel(const In
       p[4 * i4] = tp.x; p[4 * i4 + 1] = tp.y; p[4 * i4 + 2] = tp.z; p[4 * i4 + 3] = tp.w;
     }
   }
-  const float t0 = philox_uniform01(a.seed, pid, kTagTau0) * a.dt;  // sampling_utils.py:32
+  const float t0 = OD ? 0.f : philox_uniform01(a.seed, pid, kTagTau0) * a.dt;  // sampling_utils.py:32
   const int Sn = a.n_steps;
-  // BLK: element (sample s, tile t, component c, lane l) at ((s T + t) 3d + c) 128 + l ; SOA: c S N + s N + n
+  constexpr int CW = OD ? 2 * DP : 3 * DP;  // floats per emitted sample: [x, v, grad V] or (OD) [x, grad V]
+  // BLK: element (sample s, tile t, component c, lane l) at ((s T + t) CW + c) 128 + l ; SOA: c S N + s N + n
   const int64_t plane = BLK ? 128 : (int64_t)Sn * a.n;
-  const int64_t sstride = BLK ? (int64_t)gridDim.x * (3 * DP * 128) : a.n;
-  float* o = TRAJ == 0 ? nullptr : (BLK ? a.traj + ((int64_t)blockIdx.x * (3 * DP) * 128 + tid) : a.traj + n);
+  const int64_t sstride = BLK ? (int64_t)gridDim.x * (CW * 128) : a.n;
+  float* o = TRAJ == 0 ? nullptr : (BLK ? a.traj + ((int64_t)blockIdx.x * CW * 128 + tid) : a.traj + n);
+  // OD: S steps, and with a trajectory one more drift evaluation (s == S) for the last sample
+  const int s_end = OD ? Sn + (TRAJ != 0 ? 1 : 0) : Sn + 1;
 
   auto wait_commit = [&]() {
     if (!*dead_p) {
@@ -197,8 +212,8 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_mlp_tc_kernel(const In
   };
 
 #pragma unroll 1
-  for (int s = 0; s <= Sn; ++s) {
-    const float h = (s == 0) ? t0 : ((s == Sn) ? a.dt - t0 : a.dt);  // sampling_utils.py:33,45-46
+  for (int s = 0; OD ? s < s_end : s <= Sn; ++s) {
+    const float h = OD ? a.dt : ((s == 0) ? t0 : ((s == Sn) ? a.dt - t0 : a.dt));  // sampling_utils.py:33,45-46
     const float sq = sqrtf(h) * 1.41421356237309515f;
     const float dmp = 1.f - a.gamma * h;
 
@@ -218,12 +233,18 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_mlp_tc_kernel(const In
     }
     __syncwarp();
     // the drift-independent part of the kick while F0 runs: p <- p (1 - gamma h) + sqrt(2h) xi
+    // (OD: x <- x + sqrt(2h) xi; x is in the activation tile already)
+    if (!OD || s < Sn) {
 #pragma unroll
-    for (int j = 0; j < DP / 4; ++j) {
-      float r4[4];
-      philox_normal4_rk(a.rk, pid, a.step_offset + (uint32_t)s, (uint32_t)j, r4);
+      for (int j = 0; j < DP / 4; ++j) {
+        float r4[4];
+        philox_normal4_rk(a.rk, pid, a.step_offset + (uint32_t)s, (uint32_t)j, r4);
 #pragma unroll
-      for (int k = 0; k < 4; ++k) p[4 * j + k] = fmaf(sq, r4[k], p[4 * j + k] * dmp);
+        for (int k = 0; k < 4; ++k) {
+          if constexpr (OD) q[4 * j + k] = fmaf(sq, r4[k], q[4 * j + k]);
+          else p[4 * j + k] = fmaf(sq, r4[k], p[4 * j + k] * dmp);
+        }
+      }
     }
     wait_commit();
 
@@ -318,27 +339,43 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_mlp_tc_kernel(const In
     for (int c = 0; c < DK / 16; ++c) tm_ld16(t_row + 64 + 16 * c, g + 16 * c);
     tm_wait_ld();
     if constexpr (TRAJ != 0) {
-      float* og = (s == 0 ? o : o - sstride) + 2 * DP * plane;
+      float* og = (s == 0 ? o : o - sstride) + (OD ? DP : 2 * DP) * plane;
 #pragma unroll
       for (int k = 0; k < DP; ++k) __stcs(og + k * plane, g[k]);
     }
-#pragma unroll
-    for (int k = 0; k < DP; ++k) {
-      p[k] = fmaf(-h, g[k], p[k]);
-      q[k] = fmaf(h, p[k], q[k]);
-    }
-    if constexpr (TRAJ != 0) {
+    if constexpr (OD) {  // x' = (x + sqrt(2h) xi) - h grad V_theta(x)
       if (s < Sn) {
 #pragma unroll
-        for (int k = 0; k < DP; ++k) {
-          __stcs(o + k * plane, q[k]);
-          __stcs(o + (DP + k) * plane, p[k]);
+        for (int k = 0; k < DP; ++k) q[k] = fmaf(-h, g[k], q[k]);
+        if constexpr (TRAJ != 0) {
+#pragma unroll
+          for (int k = 0; k < DP; ++k) __stcs(o + k * plane, q[k]);
         }
       }
-      o += sstride;
+      if constexpr (TRAJ != 0) o += sstride;
+    } else {
+#pragma unroll
+      for (int k = 0; k < DP; ++k) {
+        p[k] = fmaf(-h, g[k], p[k]);
+        q[k] = fmaf(h, p[k], q[k]);
+      }
+      if constexpr (TRAJ != 0) {
+        if (s < Sn) {
+#pragma unroll
+          for (int k = 0; k < DP; ++k) {
+            __stcs(o + k * plane, q[k]);
+            __stcs(o + (DP + k) * plane, p[k]);
+          }
+        }
+        o += sstride;
+      }
     }
   }
-  {
+  if constexpr (OD) {
+    float4* zl = reinterpret_cast<float4*>(a.z_last + n * DP);
+#pragma unroll
+    for (int i4 = 0; i4 < DP / 4; ++i4) zl[i4] = make_float4(q[4 * i4], q[4 * i4 + 1], q[4 * i4 + 2], q[4 * i4 + 3]);
+  } else {
     float4* zl = reinterpret_cast<float4*>(a.z_last + n * (2 * DP));
 #pragma unroll
     for (int i4 = 0; i4 < DP / 4; ++i4) {
@@ -351,14 +388,14 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_mlp_tc_kernel(const In
   if (warp == 0) tmem_dealloc(tbase, S::TMEM_COLS);
 }
 
-template <int DP>
+template <int DP, bool OD>
 static int launch(const IntegrateArgs& a, int* status, cudaStream_t st) {
   using S = Cfg<DP>;
   constexpr int MINB = DP >= 16 ? 3 : 4;  // 128 TMEM columns per CTA: at most 4 CTAs per SM (d = 16 spills at 4)
   void (*kern)(const IntegrateArgs, int*);
-  if (a.traj == nullptr) kern = kl_integrate_mlp_tc_kernel<DP, 0, MINB>;
-  else if (a.traj_layout == PDEIP_TRAJ_BLOCK128) kern = kl_integrate_mlp_tc_kernel<DP, 1, MINB>;
-  else kern = kl_integrate_mlp_tc_kernel<DP, 2, MINB>;
+  if (a.traj == nullptr) kern = kl_integrate_mlp_tc_kernel<DP, 0, MINB, OD>;
+  else if (a.traj_layout == PDEIP_TRAJ_BLOCK128) kern = kl_integrate_mlp_tc_kernel<DP, 1, MINB, OD>;
+  else kern = kl_integrate_mlp_tc_kernel<DP, 2, MINB, OD>;
   PDEIP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL));
   kern<<<(unsigned)((a.n + 127) / 128), 128, S::TOTAL, st>>>(a, status);
   PDEIP_LAUNCH_OK();
@@ -380,9 +417,27 @@ int launch_integrate_mlp_tensor(const IntegrateArgs& a, cudaStream_t st) {
   int* status = tensor_status_word();
   PDEIP_REQUIRE(status != nullptr, PDEIP_ERR_CUDA, "cannot allocate the tensor-path status word");
   status += 1;  // word 1: integrator
-  if (a.d == 8) return imlp::launch<8>(a, status, st);
-  if (a.d == 16) return imlp::launch<16>(a, status, st);
-  return imlp::launch<32>(a, status, st);
+  if (a.d == 8) return imlp::launch<8, false>(a, status, st);
+  if (a.d == 16) return imlp::launch<16, false>(a, status, st);
+  return imlp::launch<32, false>(a, status, st);
+}
+
+// the overdamped arguments come on the UNIFORM schedule without tau0 (pdeip_overdamped_integrate_model)
+bool overdamped_mlp_tensor_ok(const IntegrateArgs& a) {
+  return a.layers == 2 && (a.d == 8 || a.d == 16 || a.d == 32) && !a.noise && a.z_last &&
+         a.state_layout == PDEIP_LAYOUT_AOS && a.emit_every == 1 && a.emit_offset == 0 &&
+         (a.traj == nullptr ||
+          (a.emit_drift && (a.traj_layout == PDEIP_TRAJ_BLOCK128 || a.traj_layout == PDEIP_TRAJ_TIME_SOA))) &&
+         getenv("PDEIP_NO_TC_INTEGRATOR") == nullptr;
+}
+
+int launch_overdamped_mlp_tensor(const IntegrateArgs& a, cudaStream_t st) {
+  int* status = tensor_status_word();
+  PDEIP_REQUIRE(status != nullptr, PDEIP_ERR_CUDA, "cannot allocate the tensor-path status word");
+  status += 1;  // word 1: integrator
+  if (a.d == 8) return imlp::launch<8, true>(a, status, st);
+  if (a.d == 16) return imlp::launch<16, true>(a, status, st);
+  return imlp::launch<32, true>(a, status, st);
 }
 
 }  // namespace pdeip

@@ -130,6 +130,70 @@ def kl_integrate_model(z0: torch.Tensor, n_steps: int, dt: float, gamma: float, 
     return z_last, traj, tau
 
 
+def _od_buffers(x0, n_steps, noise, state_layout, traj_layout, want_traj, emit_every, emit_offset, emit_drift):
+    """Checked inputs and the outputs of one K1-OD call: (x0, n, d, noise, x_last, traj|None)."""
+    x0 = _f32(x0, "x0")
+    if state_layout == L.LAYOUT_AOS:
+        n, d = x0.shape
+    else:
+        d, n = x0.shape
+    noise = _f32(noise, "noise", allow_none=True)
+    if noise is not None and tuple(noise.shape) != (n, n_steps, d):
+        raise PdeipError(f"noise must have shape {(n, n_steps, d)}, got {tuple(noise.shape)}")
+    s_emit = (n_steps - emit_offset + emit_every - 1) // emit_every
+    traj = None
+    if want_traj:
+        width = 2 * d if emit_drift else d
+        shape = {L.TRAJ_PARTICLE_MAJOR: (n, s_emit, width), L.TRAJ_TIME_MAJOR: (s_emit, n, width),
+                 L.TRAJ_TIME_SOA: (width, s_emit, n), L.TRAJ_BLOCK128: (s_emit, n // 128, width, 128)}[traj_layout]
+        if traj_layout == L.TRAJ_BLOCK128 and n % 128:
+            raise PdeipError(f"TRAJ_BLOCK128 needs n % 128 == 0, got n={n}")
+        traj = torch.empty(shape, device=x0.device, dtype=torch.float32)
+    return x0, n, d, noise, torch.empty_like(x0), traj
+
+
+def overdamped_integrate(x0: torch.Tensor, n_steps: int, dt: float, drift_kind: int,
+                         drift_params: Optional[torch.Tensor] = None, n_gaussian: int = 0, sigma: float = 1.0,
+                         noise: Optional[torch.Tensor] = None, seed: int = 0, particle_offset: int = 0,
+                         step_offset: int = 0, state_layout: int = L.LAYOUT_AOS,
+                         traj_layout: int = L.TRAJ_PARTICLE_MAJOR, want_traj: bool = True, emit_every: int = 1,
+                         emit_offset: int = 0, emit_drift: bool = False, path: int = L.PATH_FP32,
+                         ) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+    """pdeip_overdamped_integrate: n_steps overdamped Langevin steps x' = x - dt grad U(x) + sqrt(2 dt) xi.
+    x0: [N,d] (AOS) or [d,N] (SOA).  noise: injected normals [N, n_steps, d], else Philox.  Returns (x_last,
+    traj|None); with emit_drift every trajectory sample is [x, grad U(x)] (2d components)."""
+    x0, n, d, noise, x_last, traj = _od_buffers(x0, n_steps, noise, state_layout, traj_layout, want_traj, emit_every,
+                                                emit_offset, emit_drift)
+    drift_params = _f32(drift_params, "drift_params", allow_none=True)
+    _ops.overdamped_integrate(x0, x_last, traj, n, d, n_steps, float(dt), drift_kind, drift_params, n_gaussian,
+                              float(sigma), noise, as_i64(seed), as_i64(particle_offset), step_offset, state_layout,
+                              traj_layout, emit_every, emit_offset, 1 if emit_drift else 0, path)
+    launch_counter["n"] += 1
+    return x_last, traj
+
+
+def overdamped_integrate_model(x0: torch.Tensor, n_steps: int, dt: float, spec: "ModelSpec", params: torch.Tensor,
+                               noise: Optional[torch.Tensor] = None, seed: int = 0, particle_offset: int = 0,
+                               step_offset: int = 0, state_layout: int = L.LAYOUT_AOS,
+                               traj_layout: int = L.TRAJ_PARTICLE_MAJOR, want_traj: bool = True, emit_every: int = 1,
+                               emit_offset: int = 0, emit_drift: bool = False, path: int = L.PATH_FP32,
+                               ) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+    """pdeip_overdamped_integrate_model: overdamped_integrate with grad U = grad V_theta of the hypothesis model `spec`
+    at the flat parameters `params`.  PATH_TENSOR runs the MLP 32 x 2 drift on tcgen05 inside its envelope (pdeip.h)."""
+    x0, n, d, noise, x_last, traj = _od_buffers(x0, n_steps, noise, state_layout, traj_layout, want_traj, emit_every,
+                                                emit_offset, emit_drift)
+    params = _f32(params, "params")
+    if d != spec.d or params.numel() != spec.num_params:
+        raise PdeipError(f"shape mismatch: the state has d={d}, params has {params.numel()} entries (expected "
+                         f"d={spec.d}, {spec.num_params} params)")
+    _ops.overdamped_integrate_model(x0, x_last, traj, n, d, n_steps, float(dt), spec.kind, params, spec.hidden,
+                                    spec.layers, spec.n_gaussian, noise, as_i64(seed), as_i64(particle_offset),
+                                    step_offset, state_layout, traj_layout, emit_every, emit_offset,
+                                    1 if emit_drift else 0, path)
+    launch_counter["n"] += 1
+    return x_last, traj
+
+
 def philox_normals(n: int, n_draws: int, d: int, seed: int, particle_offset: int = 0, step_offset: int = 0,
                    device="cuda") -> torch.Tensor:
     out = torch.empty((n, n_draws, d), device=device, dtype=torch.float32)

@@ -8,6 +8,7 @@ nothing; `ops.py` allocates the outputs and is the only caller.  There is no CPU
 registered for device type "cuda" only, so a CPU tensor fails in the dispatcher ("no kernel for backend CPU").
 
 Replaces (reference file:line, as in pdeip.h): kl_integrate, kl_integrate_model — utils/sampling_utils.py:6-52;
+overdamped_integrate, overdamped_integrate_model — the SDE of example_problems/fokker_planck_example.py;
 gmm_value_grad — core/potential.py:32-61; model_eval — core/model.py:51-62 + utils/common_utils.py:6-14; residual_* —
 methods/consistency_instances/{kinetic_fokker_planck.py:11-69, fokker_planck.py:33-63, kinetic_mckean_vlasov.py:11-120};
 adam_l2_step — main.py:20-26 + core/trainer.py:61-70; ensemble_moments — example_problems/
@@ -71,6 +72,30 @@ def kl_integrate_model(z0: torch.Tensor, z_last: torch.Tensor, traj: Optional[to
         _p(z0), _p(z_last), _p(traj), _p(tau), n_particles, d, n_steps, dt, gamma, model_kind, _p(params), hidden,
         layers, n_gaussian, _p(noise), _p(tau0), _u64(seed), _u64(particle_offset), step_offset, schedule,
         state_layout, traj_layout, emit_every, emit_offset, emit_drift, path, _stream()), "pdeip_kl_integrate_model")
+
+
+@_op("overdamped_integrate", ("x_last", "traj"))
+def overdamped_integrate(x0: torch.Tensor, x_last: torch.Tensor, traj: Optional[torch.Tensor], n_particles: int, d: int,
+                         n_steps: int, dt: float, drift_kind: int, drift_params: Optional[torch.Tensor], n_gaussian: int,
+                         sigma: float, noise: Optional[torch.Tensor], seed: int, particle_offset: int, step_offset: int,
+                         state_layout: int, traj_layout: int, emit_every: int, emit_offset: int, emit_drift: int,
+                         path: int) -> None:
+    L.check(L.load().pdeip_overdamped_integrate(
+        _p(x0), _p(x_last), _p(traj), n_particles, d, n_steps, dt, drift_kind, _p(drift_params), n_gaussian, sigma,
+        _p(noise), _u64(seed), _u64(particle_offset), step_offset, state_layout, traj_layout, emit_every, emit_offset,
+        emit_drift, path, _stream()), "pdeip_overdamped_integrate")
+
+
+@_op("overdamped_integrate_model", ("x_last", "traj"))
+def overdamped_integrate_model(x0: torch.Tensor, x_last: torch.Tensor, traj: Optional[torch.Tensor], n_particles: int,
+                               d: int, n_steps: int, dt: float, model_kind: int, params: torch.Tensor, hidden: int,
+                               layers: int, n_gaussian: int, noise: Optional[torch.Tensor], seed: int,
+                               particle_offset: int, step_offset: int, state_layout: int, traj_layout: int,
+                               emit_every: int, emit_offset: int, emit_drift: int, path: int) -> None:
+    L.check(L.load().pdeip_overdamped_integrate_model(
+        _p(x0), _p(x_last), _p(traj), n_particles, d, n_steps, dt, model_kind, _p(params), hidden, layers, n_gaussian,
+        _p(noise), _u64(seed), _u64(particle_offset), step_offset, state_layout, traj_layout, emit_every, emit_offset,
+        emit_drift, path, _stream()), "pdeip_overdamped_integrate_model")
 
 
 @_op("meanfield_noise_sums", ("sums",))
@@ -200,7 +225,8 @@ def gaussian_sample(out: torch.Tensor, n: int, dim: int, mu: Optional[torch.Tens
                                            layout, _stream()), "pdeip_gaussian_sample")
 
 
-REGISTERED = ("kl_integrate", "kl_integrate_model", "meanfield_noise_sums", "meanfield_xbar_table", "gmm_value_grad", "linear_grad",
+REGISTERED = ("kl_integrate", "kl_integrate_model", "overdamped_integrate", "overdamped_integrate_model",
+              "meanfield_noise_sums", "meanfield_xbar_table", "gmm_value_grad", "linear_grad",
               "model_eval", "residual_begin", "residual_accumulate", "residual_finalize", "kmv_mean_grad",
               "residual_accumulate_kmv", "kmv_closure_correction", "kmv_density_terms", "adam_l2_step",
               "ensemble_moments", "gather_0T", "gaussian_sample")

@@ -1,4 +1,4 @@
-"""Mirror of utils/sampling_utils.py:25-52 on the K1 CUDA integrator."""
+"""Mirror of utils/sampling_utils.py:25-52 on the K1 CUDA integrator, and its overdamped counterpart (K1-OD)."""
 from __future__ import annotations
 
 from typing import Optional, Tuple
@@ -42,3 +42,25 @@ def underdamped_langevin_dynamics_scan(q0_p0: torch.Tensor, n_steps: int, dt: fl
     kind, params, n_gaussian, sigma = spec
     return ops.kl_integrate(q0_p0, n_steps, float(dt), float(gamma_friction), kind, params, n_gaussian=n_gaussian,
                             sigma=sigma, **common)
+
+
+def overdamped_langevin_dynamics_scan(x0: torch.Tensor, n_steps: int, dt: float, key, potential_grad, *,
+                                      noise: Optional[torch.Tensor] = None, particle_offset: int = 0,
+                                      traj_layout: int = L.TRAJ_PARTICLE_MAJOR, want_trajectory: bool = True,
+                                      path: int = L.PATH_FP32,
+                                      ) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+    """Overdamped Langevin dX = -grad U(X) dt + sqrt(2) dW, the SDE of the Fokker-Planck instance, by n_steps
+    Euler-Maruyama steps x' = x - dt grad U(x) + sqrt(2 dt) xi (pdeip_overdamped_integrate).  Returns (x_last [N,d],
+    trajectory of the n_steps samples in `traj_layout` ([N,n_steps,d] by default), or None without want_trajectory); sample s is the state after
+    step s.  `potential_grad` is what underdamped_langevin_dynamics_scan takes: the .gradient of an analytic Potential or
+    of a ModelPotential(net, params).  `key` is an integer seed (Philox(seed, particle_offset + n)); `noise` [N,n_steps,d]
+    injects the draws for parity runs."""
+    spec = drift_spec(potential_grad)
+    common = dict(noise=noise, seed=int(key), particle_offset=particle_offset, traj_layout=traj_layout,
+                  want_traj=want_trajectory, path=path)
+    if isinstance(spec[0], ops.ModelSpec):
+        model_spec, flat = spec
+        return ops.overdamped_integrate_model(x0, n_steps, float(dt), model_spec, flat, **common)
+    kind, params, n_gaussian, sigma = spec
+    return ops.overdamped_integrate(x0, n_steps, float(dt), kind, params, n_gaussian=n_gaussian, sigma=sigma,
+                                    **common)

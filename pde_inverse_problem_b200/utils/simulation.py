@@ -1,10 +1,12 @@
-"""Distribution-level validation of a fitted potential on the kinetic instances: simulate the particles under the fitted
-drift and under the true one, synchronously coupled.
+"""Distribution-level validation of a fitted potential on the kinetic and the Fokker-Planck instances: simulate the
+particles under the fitted drift and under the true one, synchronously coupled.
 
 The integrator's noise is counter-based (Philox keyed by seed, global particle id and step), so two runs from the same
 initial ensemble with the same seed share every Brownian increment and every initial time shift.  The RMS distance
 between the coupled terminal states is then an upper bound on the W2 distance between the true and the fitted terminal
-laws.  The reference has no such metric (its kinetic test_fn is commented out); this module is not wired into test_fn.
+laws.  The kinetic instances run the underdamped integrator, the Fokker-Planck instance (no `gamma_friction` in its
+configuration) the overdamped one.  The reference has no such metric (its kinetic test_fn is commented out); this module
+is not wired into test_fn.
 """
 from __future__ import annotations
 
@@ -18,7 +20,7 @@ from .. import ops
 from ..core.model import model_of
 from ..core.potential import ModelPotential
 from . import rng as jrandom
-from .sampling_utils import underdamped_langevin_dynamics_scan
+from .sampling_utils import overdamped_langevin_dynamics_scan, underdamped_langevin_dynamics_scan
 
 
 def _instance_n_steps(pde_instance) -> int:
@@ -41,30 +43,42 @@ def coupled_simulation_error(pde_instance, forward_fn, n_particles: int, rng, n_
                              path: int = L.PATH_FP32) -> Dict[str, torch.Tensor]:
     """Integrate one initial ensemble (drawn from pde_instance.distribution_initial) to the terminal time twice, with
     the same seed: under pde_instance.potential and under the fitted model `forward_fn` (= functools.partial(net.apply,
-    params), as test_fn receives it).  dt = total_evolving_time / n_steps, n_steps defaults to the instance's own.
+    params), as test_fn receives it).  dt = total_evolving_time / n_steps, n_steps defaults to the instance's own on the
+    kinetic instances; the Fokker-Planck instance has no step count of its own, so there n_steps is required.
 
     Returns 0-d CUDA tensors (no host synchronisation; every reduction is one ensemble_moments call), over the full
-    (x, v) state:
+    state ((x, v) on the kinetic instances, x on the Fokker-Planck one):
       "coupled rms distance terminal"      sqrt(mean |z_true - z_fit|^2)  (>= W2 of the two terminal laws)
       "relative mean error terminal"       |mean_fit - mean_true| / |mean_true|
       "relative covariance error terminal" |C_fit - C_true|_F / |C_true|_F
     """
     potential = getattr(pde_instance, "potential", None)
     if potential is None or not hasattr(pde_instance, "distribution_initial"):
-        raise NotImplementedError("coupled_simulation_error needs a kinetic instance with a true `potential` "
-                                  "(kinetic Fokker-Planck, GMM or OU)")
+        raise NotImplementedError("coupled_simulation_error needs an instance with a true `potential` "
+                                  "(kinetic Fokker-Planck, GMM or OU, or Fokker-Planck)")
     if not isinstance(forward_fn, functools.partial) or not forward_fn.args:
         raise NotImplementedError("forward_fn must be functools.partial(net.apply, params), as test_fn receives it")
     net, params = model_of(forward_fn), forward_fn.args[0]
-    n_steps = _instance_n_steps(pde_instance) if n_steps is None else int(n_steps)
+    overdamped = "gamma_friction" not in pde_instance.initial_configuration
+    if n_steps is None:
+        if overdamped:
+            raise ValueError("n_steps is required on the Fokker-Planck instance: its configuration has no step count")
+        n_steps = _instance_n_steps(pde_instance)
+    n_steps = int(n_steps)
     dt = float(pde_instance.total_evolving_time) / n_steps
-    gamma = float(pde_instance.initial_configuration["gamma_friction"])
     rng_init, rng_sde = jrandom.split(rng)
     z0 = pde_instance.distribution_initial.sample(n_particles, rng_init)
-    z_true, _, _ = underdamped_langevin_dynamics_scan(z0, n_steps, dt, rng_sde, potential.gradient, gamma,
+    fitted = ModelPotential(net, params).gradient
+    if overdamped:
+        z_true, _ = overdamped_langevin_dynamics_scan(z0, n_steps, dt, rng_sde, potential.gradient,
                                                       want_trajectory=False, path=path)
-    z_fit, _, _ = underdamped_langevin_dynamics_scan(z0, n_steps, dt, rng_sde, ModelPotential(net, params).gradient,
-                                                     gamma, want_trajectory=False, path=path)
+        z_fit, _ = overdamped_langevin_dynamics_scan(z0, n_steps, dt, rng_sde, fitted, want_trajectory=False, path=path)
+    else:
+        gamma = float(pde_instance.initial_configuration["gamma_friction"])
+        z_true, _, _ = underdamped_langevin_dynamics_scan(z0, n_steps, dt, rng_sde, potential.gradient, gamma,
+                                                          want_trajectory=False, path=path)
+        z_fit, _, _ = underdamped_langevin_dynamics_scan(z0, n_steps, dt, rng_sde, fitted, gamma,
+                                                         want_trajectory=False, path=path)
     _, diff_second = ops.ensemble_moments(z_true - z_fit)
     rms = torch.sqrt(torch.trace(diff_second) / n_particles)
     m_true, c_true = _mean_cov(z_true)
