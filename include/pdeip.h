@@ -166,8 +166,12 @@ int pdeip_kl_integrate_model(const float* z0, float* z_last, float* traj, float*
  * four K1 trajectory layouts with C = d components per sample, or C = 2d with emit_drift: [x, grad U(x)] (the drift
  * step s+1 evaluates anyway; the last sample takes one extra evaluation).  A PDEIP_TRAJ_BLOCK128 trajectory is directly
  * a PDEIP_LAYOUT_BLOCK128 FP point set, with PDEIP_DRIFT_IN_POINTS when the drift is emitted.
- * Drifts: PDEIP_DRIFT_NONE / _LINEAR / _GMM / _MEANFIELD, fp32 on the CUDA cores on both paths (the GMM drift has no
- * overdamped tcgen05 kernel).  PDEIP_DRIFT_MEANFIELD_TABLE encodes the underdamped mean recursion and is rejected
+ * Drifts: PDEIP_DRIFT_NONE / _LINEAR / _GMM / _MEANFIELD, fp32 on the CUDA cores (rtol 1e-5 class).  PDEIP_PATH_TENSOR
+ * with the GMM drift, d = 8, 16 or 32, 1 <= n_gaussian <= 64, Philox noise, AOS state with x_last, emit_every 1,
+ * emit_offset 0 and either traj == NULL (terminal state only, n arbitrary) or a PDEIP_TRAJ_BLOCK128 /
+ * PDEIP_TRAJ_TIME_SOA trajectory with emit_drift runs the centre contraction and the softmax-weighted centre sum on
+ * tcgen05 (K1-T-OD, bf16 hi + lo split operands, "bf16 GEMM path", rtol 1e-2 class); every other call takes the fp32
+ * kernel, bit-identical to PDEIP_PATH_FP32 (PDEIP_NO_TC_INTEGRATOR=1 forces it).  PDEIP_DRIFT_MEANFIELD_TABLE encodes the underdamped mean recursion and is rejected
  * (PDEIP_ERR_UNSUPPORTED).  Rejected before any CUDA call, with a pdeip_last_error message: unknown drift kind, path or
  * layout, NULL x0 or drift_params, n_steps < 1, bad emit_every / emit_offset (PDEIP_ERR_INVALID_ARG), BLOCK128 with
  * n % 128 != 0 (PDEIP_ERR_INVALID_ARG), d outside [1, 32] (PDEIP_ERR_UNSUPPORTED).

@@ -591,9 +591,11 @@ static int launch_integrate_model(const IntegrateArgs& a, int model_kind, int pa
 }
 
 // K1-OD: the overdamped step on the generic kernel, every analytic drift and configuration (the entry point has
-// rejected PDEIP_DRIFT_MEANFIELD_TABLE and unknown kinds)
+// rejected PDEIP_DRIFT_MEANFIELD_TABLE and unknown kinds); under PDEIP_PATH_TENSOR the GMM drift of K1-T-OD's envelope
+// (integrator_tc.cu)
 template <int DP>
-static int launch_overdamped(const IntegrateArgs& a, int drift_kind, cudaStream_t st) {
+static int launch_overdamped(const IntegrateArgs& a, int drift_kind, int path, cudaStream_t st) {
+  if (path == PDEIP_PATH_TENSOR && overdamped_tensor_ok(a, drift_kind)) return launch_overdamped_tensor(a, st);
   const unsigned grid = (unsigned)((a.n + 127) / 128);
   switch (drift_kind) {
     case PDEIP_DRIFT_NONE:
@@ -912,11 +914,11 @@ extern "C" int pdeip_overdamped_integrate(const float* x0, float* x_last, float*
   a.drift_params = drift_params;
   a.n_gaussian = n_gaussian; a.inv_sigma2 = drift_kind == PDEIP_DRIFT_GMM ? 1.0f / (sigma * sigma) : 1.0f;
   cudaStream_t st = (cudaStream_t)stream;
-  if (d <= 2) return launch_overdamped<2>(a, drift_kind, st);
-  if (d <= 4) return launch_overdamped<4>(a, drift_kind, st);
-  if (d <= 8) return launch_overdamped<8>(a, drift_kind, st);
-  if (d <= 16) return launch_overdamped<16>(a, drift_kind, st);
-  return launch_overdamped<32>(a, drift_kind, st);
+  if (d <= 2) return launch_overdamped<2>(a, drift_kind, path, st);
+  if (d <= 4) return launch_overdamped<4>(a, drift_kind, path, st);
+  if (d <= 8) return launch_overdamped<8>(a, drift_kind, path, st);
+  if (d <= 16) return launch_overdamped<16>(a, drift_kind, path, st);
+  return launch_overdamped<32>(a, drift_kind, path, st);
 }
 
 extern "C" int pdeip_overdamped_integrate_model(const float* x0, float* x_last, float* traj, int64_t n_particles,

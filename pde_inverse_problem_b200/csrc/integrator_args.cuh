@@ -40,6 +40,9 @@ struct IntegrateArgs {
 // integrator_tc.cu: GMM drift on the tensor cores (PDEIP_PATH_TENSOR)
 bool integrate_tensor_ok(const IntegrateArgs& a, int drift_kind);
 int launch_integrate_tensor(const IntegrateArgs& a, cudaStream_t st);
+// ... and its overdamped variant K1-T-OD (PDEIP_PATH_TENSOR of pdeip_overdamped_integrate)
+bool overdamped_tensor_ok(const IntegrateArgs& a, int drift_kind);
+int launch_overdamped_tensor(const IntegrateArgs& a, cudaStream_t st);
 
 // integrator_mlp_tc.cu: MLP (32 x 2) drift on the tensor cores (PDEIP_PATH_TENSOR of pdeip_kl_integrate_model)
 bool integrate_mlp_tensor_ok(const IntegrateArgs& a);

@@ -20,6 +20,13 @@
 // schedule and outputs ([S][N/128][3d][128] or [3d][S][N] trajectory with grad U, final state) as
 // kl_integrate_fast_kernel (integrator.cu).  Measured: 70.8 % (d = 32, K = 64) and 69 % (d = 8, K = 16) of the HBM copy
 // bandwidth; bound by instruction issue and MUFU together (profiles/r01_summary_tc_integrator.md).
+//
+// OD = true is the overdamped variant (K1-T-OD, PDEIP_PATH_TENSOR of pdeip_overdamped_integrate with the GMM drift):
+// the state per thread is x alone, S steps x' = (x + sqrt(2h) xi_s) - h grad U(x) with h = dt and no tau0.  The
+// registers that hold p in the kinetic step hold x + sqrt(2h) xi_s, formed while the GEMMs run, because the epilogue
+// still needs x.  An emitted sample is [x, grad U(x)] ([S][N/128][2d][128] or [2d][S][N]); a trajectory run makes one
+// more drift-only iteration (s = S: GEMMs and epilogue, no noise, no update) for the last sample's drift, and TRAJ =
+// false (OD only) writes the terminal state alone.  Same operand tiles, TMEM map, splits and status word.
 #include "common.cuh"
 #include "integrator_args.cuh"
 #include "philox.cuh"
@@ -88,9 +95,10 @@ __device__ __forceinline__ void split2(float2 ab, uint32_t& hi, uint32_t& lo) {
 }
 
 // BLK = true: trajectory in PDEIP_TRAJ_BLOCK128 ([S][N/128][3d][128]: every store of a step is base + immediate);
-// false: PDEIP_TRAJ_TIME_SOA ([3d][S][N]).
-template <int DP, int KP, bool BLK, int MINB>
+// false: PDEIP_TRAJ_TIME_SOA ([3d][S][N]).  OD: the overdamped step (see above); TRAJ = false: no trajectory (OD only).
+template <int DP, int KP, bool BLK, int MINB, bool OD = false, bool TRAJ = true>
 __global__ void __launch_bounds__(128, MINB) kl_integrate_tc_kernel(const IntegrateArgs a, int* status) {
+  static_assert(TRAJ || OD, "a kinetic launch always writes its trajectory");
   using S = Cfg<DP, KP>;
   extern __shared__ __align__(128) uint8_t sm[];
   const int tid = threadIdx.x, warp = tid >> 5;
@@ -164,8 +172,15 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc_kernel(const Integr
   const int64_t n_raw = (int64_t)blockIdx.x * 128 + tid;
   const int64_t n = n_raw < a.n ? n_raw : a.n - 1;
   const uint64_t pid = a.particle_offset + (uint64_t)n;
-  float2 q[DP / 2], p[DP / 2];
-  {
+  float2 q[DP / 2], p[DP / 2];  // OD: q = x, p = x + sqrt(2h) xi of the current step
+  if constexpr (OD) {
+    const float4* z4 = reinterpret_cast<const float4*>(a.z0 + n * DP);
+#pragma unroll
+    for (int i4 = 0; i4 < DP / 4; ++i4) {
+      const float4 tq = z4[i4];
+      q[2 * i4] = make_float2(tq.x, tq.y); q[2 * i4 + 1] = make_float2(tq.z, tq.w);
+    }
+  } else {
     const float4* z4 = reinterpret_cast<const float4*>(a.z0 + n * (2 * DP));
 #pragma unroll
     for (int i4 = 0; i4 < DP / 4; ++i4) {
@@ -174,13 +189,16 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc_kernel(const Integr
       p[2 * i4] = make_float2(tp.x, tp.y); p[2 * i4 + 1] = make_float2(tp.z, tp.w);
     }
   }
-  const float t0 = philox_uniform01(a.seed, pid, kTagTau0) * a.dt;  // sampling_utils.py:32
+  const float t0 = OD ? 0.f : philox_uniform01(a.seed, pid, kTagTau0) * a.dt;  // sampling_utils.py:32
   const int Sn = a.n_steps;
-  // BLK: element (sample s, tile t, component c, lane l) at ((s T + t) 3d + c) 128 + l ; else c S N + s N + n
+  constexpr int CW = OD ? 2 * DP : 3 * DP;  // floats per emitted sample: [x, v, grad U] or (OD) [x, grad U]
+  // BLK: element (sample s, tile t, component c, lane l) at ((s T + t) CW + c) 128 + l ; else c S N + s N + n
   const int64_t plane = BLK ? 128 : (int64_t)Sn * a.n;               // floats between components of a sample
-  const int64_t sstride = BLK ? (int64_t)gridDim.x * (3 * DP * 128) : a.n;  // floats between samples
-  float* o = BLK ? a.traj + ((int64_t)blockIdx.x * (3 * DP) * 128 + tid) : a.traj + n;  // sample 0, component 0
+  const int64_t sstride = BLK ? (int64_t)gridDim.x * (CW * 128) : a.n;  // floats between samples
+  float* o = !TRAJ ? nullptr : (BLK ? a.traj + ((int64_t)blockIdx.x * CW * 128 + tid) : a.traj + n);  // sample 0, component 0
   const float rcs = 1.0f / cs;
+  // OD: S steps, and with a trajectory one more drift-only iteration (s = S) for the last sample's drift
+  const int s_end = OD ? Sn + (TRAJ ? 1 : 0) : Sn + 1;
 
   auto wait_commit = [&]() {
     if (!*dead_p) {
@@ -193,20 +211,27 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc_kernel(const Integr
     fence_after_sync();
   };
   // p <- p (1 - gamma h) + sqrt(2h) xi for coordinate blocks [j0, j1) (4 coordinates each): the drift-independent part
+  // (OD: p <- x + sqrt(2h) xi; the drift-only iteration s = S draws nothing)
   auto kick = [&](int s, float dmp, float sq, int j0, int j1) {
+    if (OD && s == Sn) return;
     const float2 dmp2 = make_float2(dmp, dmp), sq2 = make_float2(sq, sq);
 #pragma unroll
     for (int j = j0; j < j1; ++j) {
       float r4[4];
       philox_normal4_rk(a.rk, pid, a.step_offset + (uint32_t)s, (uint32_t)j, r4);
-      p[2 * j] = __ffma2_rn(sq2, make_float2(r4[0], r4[1]), __fmul2_rn(p[2 * j], dmp2));
-      p[2 * j + 1] = __ffma2_rn(sq2, make_float2(r4[2], r4[3]), __fmul2_rn(p[2 * j + 1], dmp2));
+      if constexpr (OD) {
+        p[2 * j] = __ffma2_rn(sq2, make_float2(r4[0], r4[1]), q[2 * j]);
+        p[2 * j + 1] = __ffma2_rn(sq2, make_float2(r4[2], r4[3]), q[2 * j + 1]);
+      } else {
+        p[2 * j] = __ffma2_rn(sq2, make_float2(r4[0], r4[1]), __fmul2_rn(p[2 * j], dmp2));
+        p[2 * j + 1] = __ffma2_rn(sq2, make_float2(r4[2], r4[3]), __fmul2_rn(p[2 * j + 1], dmp2));
+      }
     }
   };
 
 #pragma unroll 1
-  for (int s = 0; s <= Sn; ++s) {
-    const float h = (s == 0) ? t0 : ((s == Sn) ? a.dt - t0 : a.dt);  // sampling_utils.py:33,45-46
+  for (int s = 0; OD ? s < s_end : s <= Sn; ++s) {
+    const float h = OD ? a.dt : ((s == 0) ? t0 : ((s == Sn) ? a.dt - t0 : a.dt));  // sampling_utils.py:33,45-46
     const float sq = sqrtf(h) * 1.41421356237309515f;
     const float dmp = 1.f - a.gamma * h;
 
@@ -296,7 +321,7 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc_kernel(const Integr
     const float rn = -rcs / (se2.x + se2.y);
     const float2 rn2 = make_float2(rn, rn), is2 = make_float2(a.inv_sigma2, a.inv_sigma2);
     const float2 nh2 = make_float2(-h, -h), h2 = make_float2(h, h);
-    float* og = (s == 0 ? o : o - sstride) + 2 * DP * plane;
+    float* og = (s == 0 ? o : o - sstride) + (OD ? DP : 2 * DP) * plane;
 #pragma unroll
     for (int c = 0; c < DP / 16; ++c) {
       float acc[16];
@@ -306,26 +331,34 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc_kernel(const Integr
       for (int i = 0; i < 8; ++i) {
         const int k = 8 * c + i;
         const float2 g = __fmul2_rn(__ffma2_rn(make_float2(acc[2 * i], acc[2 * i + 1]), rn2, q[k]), is2);
-        if constexpr (BLK) {
-          __stcs(og + (2 * k) * 128, g.x);
-          __stcs(og + (2 * k + 1) * 128, g.y);
-        } else {
-          __stcs(og, g.x);
-          __stcs(og + plane, g.y);
-          og += 2 * plane;
+        if constexpr (TRAJ) {
+          if constexpr (BLK) {
+            __stcs(og + (2 * k) * 128, g.x);
+            __stcs(og + (2 * k + 1) * 128, g.y);
+          } else {
+            __stcs(og, g.x);
+            __stcs(og + plane, g.y);
+            og += 2 * plane;
+          }
         }
-        p[k] = __ffma2_rn(nh2, g, p[k]);
-        q[k] = __ffma2_rn(h2, p[k], q[k]);
+        if constexpr (OD) {  // x' = (x + sqrt(2h) xi) - h grad U(x)
+          if (s < Sn) q[k] = __ffma2_rn(nh2, g, p[k]);
+        } else {
+          p[k] = __ffma2_rn(nh2, g, p[k]);
+          q[k] = __ffma2_rn(h2, p[k], q[k]);
+        }
       }
     }
-    if (s < Sn) {
+    if (TRAJ && s < Sn) {  // the state as sample s: [x, v] (OD: x; its drift follows in the next iteration)
       if constexpr (BLK) {
 #pragma unroll
         for (int i = 0; i < DP / 2; ++i) {
           __stcs(o + (2 * i) * 128, q[i].x);
           __stcs(o + (2 * i + 1) * 128, q[i].y);
-          __stcs(o + (DP + 2 * i) * 128, p[i].x);
-          __stcs(o + (DP + 2 * i + 1) * 128, p[i].y);
+          if constexpr (!OD) {
+            __stcs(o + (DP + 2 * i) * 128, p[i].x);
+            __stcs(o + (DP + 2 * i + 1) * 128, p[i].y);
+          }
         }
       } else {
         float* w = o;
@@ -335,17 +368,23 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc_kernel(const Integr
           __stcs(w + plane, q[i].y);
           w += 2 * plane;
         }
+        if constexpr (!OD) {
 #pragma unroll
-        for (int i = 0; i < DP / 2; ++i) {
-          __stcs(w, p[i].x);
-          __stcs(w + plane, p[i].y);
-          w += 2 * plane;
+          for (int i = 0; i < DP / 2; ++i) {
+            __stcs(w, p[i].x);
+            __stcs(w + plane, p[i].y);
+            w += 2 * plane;
+          }
         }
       }
     }
-    o += sstride;
+    if constexpr (TRAJ) o += sstride;
   }
-  {
+  if constexpr (OD) {
+    float4* zl = reinterpret_cast<float4*>(a.z_last + n * DP);
+#pragma unroll
+    for (int i4 = 0; i4 < DP / 4; ++i4) zl[i4] = make_float4(q[2 * i4].x, q[2 * i4].y, q[2 * i4 + 1].x, q[2 * i4 + 1].y);
+  } else {
     float4* zl = reinterpret_cast<float4*>(a.z_last + n * (2 * DP));
 #pragma unroll
     for (int i4 = 0; i4 < DP / 4; ++i4) {
@@ -377,8 +416,9 @@ struct Cfg8 {
 #ifndef PDEIP_ITC8_MINB
 #define PDEIP_ITC8_MINB 8
 #endif
-template <int KP, bool BLK, int MINB>
+template <int KP, bool BLK, int MINB, bool OD = false, bool TRAJ = true>
 __global__ void __launch_bounds__(128, MINB) kl_integrate_tc8_kernel(const IntegrateArgs a, int* status) {
+  static_assert(TRAJ || OD, "a kinetic launch always writes its trajectory");
   using S = Cfg8<KP>;
   constexpr int DP = 8;
   extern __shared__ __align__(128) uint8_t sm[];
@@ -434,19 +474,25 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc8_kernel(const Integ
   const int64_t n_raw = (int64_t)blockIdx.x * 128 + tid;
   const int64_t n = n_raw < a.n ? n_raw : a.n - 1;  // ragged last tile: repeat the last particle (see above)
   const uint64_t pid = a.particle_offset + (uint64_t)n;
-  float2 q[4], p[4];
-  {
+  float2 q[4], p[4];  // OD: q = x, p = x + sqrt(2h) xi of the current step
+  if constexpr (OD) {
+    const float4* z4 = reinterpret_cast<const float4*>(a.z0 + n * 8);
+    const float4 q0 = z4[0], q1 = z4[1];
+    q[0] = make_float2(q0.x, q0.y); q[1] = make_float2(q0.z, q0.w); q[2] = make_float2(q1.x, q1.y); q[3] = make_float2(q1.z, q1.w);
+  } else {
     const float4* z4 = reinterpret_cast<const float4*>(a.z0 + n * 16);
     const float4 q0 = z4[0], q1 = z4[1], p0 = z4[2], p1 = z4[3];
     q[0] = make_float2(q0.x, q0.y); q[1] = make_float2(q0.z, q0.w); q[2] = make_float2(q1.x, q1.y); q[3] = make_float2(q1.z, q1.w);
     p[0] = make_float2(p0.x, p0.y); p[1] = make_float2(p0.z, p0.w); p[2] = make_float2(p1.x, p1.y); p[3] = make_float2(p1.z, p1.w);
   }
-  const float t0 = philox_uniform01(a.seed, pid, kTagTau0) * a.dt;  // sampling_utils.py:32
+  const float t0 = OD ? 0.f : philox_uniform01(a.seed, pid, kTagTau0) * a.dt;  // sampling_utils.py:32
   const int Sn = a.n_steps;
+  constexpr int CW = OD ? 2 * DP : 3 * DP;  // floats per emitted sample
   const int64_t plane = BLK ? 128 : (int64_t)Sn * a.n;
-  const int64_t sstride = BLK ? (int64_t)gridDim.x * (3 * DP * 128) : a.n;
-  float* o = BLK ? a.traj + ((int64_t)blockIdx.x * (3 * DP) * 128 + tid) : a.traj + n;
+  const int64_t sstride = BLK ? (int64_t)gridDim.x * (CW * 128) : a.n;
+  float* o = !TRAJ ? nullptr : (BLK ? a.traj + ((int64_t)blockIdx.x * CW * 128 + tid) : a.traj + n);
   const float rcs = 1.0f / cs;
+  const int s_end = OD ? Sn + (TRAJ ? 1 : 0) : Sn + 1;  // OD: + the drift-only iteration of a trajectory run
 
   auto wait_commit = [&]() {
     if (!*dead_p) {
@@ -459,16 +505,22 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc8_kernel(const Integ
     fence_after_sync();
   };
   auto kick = [&](int s, float dmp, float sq, int j) {  // p <- p (1 - gamma h) + sqrt(2h) xi, coordinates 4j .. 4j+3
+    if (OD && s == Sn) return;                          // (OD: p <- x + sqrt(2h) xi; none at s = S)
     const float2 dmp2 = make_float2(dmp, dmp), sq2 = make_float2(sq, sq);
     float r4[4];
     philox_normal4_rk(a.rk, pid, a.step_offset + (uint32_t)s, (uint32_t)j, r4);
-    p[2 * j] = __ffma2_rn(sq2, make_float2(r4[0], r4[1]), __fmul2_rn(p[2 * j], dmp2));
-    p[2 * j + 1] = __ffma2_rn(sq2, make_float2(r4[2], r4[3]), __fmul2_rn(p[2 * j + 1], dmp2));
+    if constexpr (OD) {
+      p[2 * j] = __ffma2_rn(sq2, make_float2(r4[0], r4[1]), q[2 * j]);
+      p[2 * j + 1] = __ffma2_rn(sq2, make_float2(r4[2], r4[3]), q[2 * j + 1]);
+    } else {
+      p[2 * j] = __ffma2_rn(sq2, make_float2(r4[0], r4[1]), __fmul2_rn(p[2 * j], dmp2));
+      p[2 * j + 1] = __ffma2_rn(sq2, make_float2(r4[2], r4[3]), __fmul2_rn(p[2 * j + 1], dmp2));
+    }
   };
 
 #pragma unroll 1
-  for (int s = 0; s <= Sn; ++s) {
-    const float h = (s == 0) ? t0 : ((s == Sn) ? a.dt - t0 : a.dt);  // sampling_utils.py:33,45-46
+  for (int s = 0; OD ? s < s_end : s <= Sn; ++s) {
+    const float h = OD ? a.dt : ((s == 0) ? t0 : ((s == Sn) ? a.dt - t0 : a.dt));  // sampling_utils.py:33,45-46
     const float sq = sqrtf(h) * 1.41421356237309515f;
     const float dmp = 1.f - a.gamma * h;
     {
@@ -546,29 +598,41 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc8_kernel(const Integ
     const float rn = -rcs / (se2.x + se2.y);
     const float2 rn2 = make_float2(rn, rn), is2 = make_float2(a.inv_sigma2, a.inv_sigma2);
     const float2 nh2 = make_float2(-h, -h), h2 = make_float2(h, h);
-    float* og = (s == 0 ? o : o - sstride) + 2 * DP * plane;
+    float* og = (s == 0 ? o : o - sstride) + (OD ? DP : 2 * DP) * plane;
     float acc[8];
     tmem_ld8(t_acc, acc);
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
       const float2 g = __fmul2_rn(__ffma2_rn(make_float2(acc[2 * k], acc[2 * k + 1]), rn2, q[k]), is2);
-      __stcs(og + (2 * k) * plane, g.x);
-      __stcs(og + (2 * k + 1) * plane, g.y);
-      p[k] = __ffma2_rn(nh2, g, p[k]);
-      q[k] = __ffma2_rn(h2, p[k], q[k]);
+      if constexpr (TRAJ) {
+        __stcs(og + (2 * k) * plane, g.x);
+        __stcs(og + (2 * k + 1) * plane, g.y);
+      }
+      if constexpr (OD) {  // x' = (x + sqrt(2h) xi) - h grad U(x)
+        if (s < Sn) q[k] = __ffma2_rn(nh2, g, p[k]);
+      } else {
+        p[k] = __ffma2_rn(nh2, g, p[k]);
+        q[k] = __ffma2_rn(h2, p[k], q[k]);
+      }
     }
-    if (s < Sn) {
+    if (TRAJ && s < Sn) {
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
         __stcs(o + (2 * i) * plane, q[i].x);
         __stcs(o + (2 * i + 1) * plane, q[i].y);
-        __stcs(o + (DP + 2 * i) * plane, p[i].x);
-        __stcs(o + (DP + 2 * i + 1) * plane, p[i].y);
+        if constexpr (!OD) {
+          __stcs(o + (DP + 2 * i) * plane, p[i].x);
+          __stcs(o + (DP + 2 * i + 1) * plane, p[i].y);
+        }
       }
     }
-    o += sstride;
+    if constexpr (TRAJ) o += sstride;
   }
-  {
+  if constexpr (OD) {
+    float4* zl = reinterpret_cast<float4*>(a.z_last + n * 8);
+    zl[0] = make_float4(q[0].x, q[0].y, q[1].x, q[1].y);
+    zl[1] = make_float4(q[2].x, q[2].y, q[3].x, q[3].y);
+  } else {
     float4* zl = reinterpret_cast<float4*>(a.z_last + n * 16);
     zl[0] = make_float4(q[0].x, q[0].y, q[1].x, q[1].y);
     zl[1] = make_float4(q[2].x, q[2].y, q[3].x, q[3].y);
@@ -580,34 +644,56 @@ __global__ void __launch_bounds__(128, MINB) kl_integrate_tc8_kernel(const Integ
   if (warp == 0) tmem_dealloc(tbase, S::TMEM_COLS);
 }
 
+// CTAs per SM the overdamped instances are sized for (fixed; the PDEIP_ITC*_MINB knobs tune the kinetic instances):
+// the kinetic defaults where ptxas fits them without a stack frame.  At d = 8 a budget of 8 CTAs (64 registers) needs
+// one, so the trajectory instances take 6.  The terminal-only ones need one at 6 (K >= 48) and at 5 (K = 64): they take
+// 5, and 4 at K = 64, where a CTA's 128 TMEM columns allow no more than 4 CTAs per SM anyway.
+constexpr int kOdMinb16 = 3, kOdMinb32 = 3, kOdMinb8Traj = 6;
 template <int KP>
+constexpr int kOdMinb8Terminal = KP == 64 ? 4 : 5;
+
+template <int KP, bool OD>
 static int launch8(const IntegrateArgs& a, int* status, cudaStream_t st) {
   using S = Cfg8<KP>;
   const int64_t grid = (a.n + 127) / 128;
-  const char* mb = getenv("PDEIP_ITC8_MINB");  // tuning knob: CTAs per SM the register budget is sized for
-  const bool eight = mb ? (mb[0] == '8') : (PDEIP_ITC8_MINB == 8);
   void (*kern)(const IntegrateArgs, int*);
-  if (a.traj_layout == PDEIP_TRAJ_BLOCK128)
-    kern = eight ? kl_integrate_tc8_kernel<KP, true, 8> : kl_integrate_tc8_kernel<KP, true, 6>;
-  else
-    kern = eight ? kl_integrate_tc8_kernel<KP, false, 8> : kl_integrate_tc8_kernel<KP, false, 6>;
+  if constexpr (OD) {
+    constexpr int MB = kOdMinb8Traj;
+    if (a.traj == nullptr) kern = kl_integrate_tc8_kernel<KP, false, kOdMinb8Terminal<KP>, true, false>;
+    else if (a.traj_layout == PDEIP_TRAJ_BLOCK128) kern = kl_integrate_tc8_kernel<KP, true, MB, true>;
+    else kern = kl_integrate_tc8_kernel<KP, false, MB, true>;
+  } else {
+    const char* mb = getenv("PDEIP_ITC8_MINB");  // tuning knob: CTAs per SM the register budget is sized for
+    const bool eight = mb ? (mb[0] == '8') : (PDEIP_ITC8_MINB == 8);
+    if (a.traj_layout == PDEIP_TRAJ_BLOCK128)
+      kern = eight ? kl_integrate_tc8_kernel<KP, true, 8> : kl_integrate_tc8_kernel<KP, true, 6>;
+    else
+      kern = eight ? kl_integrate_tc8_kernel<KP, false, 8> : kl_integrate_tc8_kernel<KP, false, 6>;
+  }
   PDEIP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL));
   kern<<<(unsigned)grid, 128, S::TOTAL, st>>>(a, status);
   PDEIP_LAUNCH_OK();
   return PDEIP_OK;
 }
 
-template <int DP, int KP>
+template <int DP, int KP, bool OD>
 static int launch(const IntegrateArgs& a, int* status, cudaStream_t st) {
   using S = Cfg<DP, KP>;
   const int64_t grid = (a.n + 127) / 128;
-  const char* mb = getenv("PDEIP_ITC_MINB");  // tuning knob: CTAs per SM the register budget is sized for
-  const bool four = mb ? (mb[0] == '4') : (PDEIP_ITC_MINB == 4);
   void (*kern)(const IntegrateArgs, int*);
-  if (a.traj_layout == PDEIP_TRAJ_BLOCK128)
-    kern = four ? kl_integrate_tc_kernel<DP, KP, true, 4> : kl_integrate_tc_kernel<DP, KP, true, 3>;
-  else
-    kern = four ? kl_integrate_tc_kernel<DP, KP, false, 4> : kl_integrate_tc_kernel<DP, KP, false, 3>;
+  if constexpr (OD) {
+    constexpr int MB = DP == 32 ? kOdMinb32 : kOdMinb16;
+    if (a.traj == nullptr) kern = kl_integrate_tc_kernel<DP, KP, false, MB, true, false>;
+    else if (a.traj_layout == PDEIP_TRAJ_BLOCK128) kern = kl_integrate_tc_kernel<DP, KP, true, MB, true>;
+    else kern = kl_integrate_tc_kernel<DP, KP, false, MB, true>;
+  } else {
+    const char* mb = getenv("PDEIP_ITC_MINB");  // tuning knob: CTAs per SM the register budget is sized for
+    const bool four = mb ? (mb[0] == '4') : (PDEIP_ITC_MINB == 4);
+    if (a.traj_layout == PDEIP_TRAJ_BLOCK128)
+      kern = four ? kl_integrate_tc_kernel<DP, KP, true, 4> : kl_integrate_tc_kernel<DP, KP, true, 3>;
+    else
+      kern = four ? kl_integrate_tc_kernel<DP, KP, false, 4> : kl_integrate_tc_kernel<DP, KP, false, 3>;
+  }
   PDEIP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::TOTAL));
   kern<<<(unsigned)grid, 128, S::TOTAL, st>>>(a, status);
   PDEIP_LAUNCH_OK();
@@ -623,27 +709,46 @@ bool integrate_tensor_ok(const IntegrateArgs& a, int drift_kind) {
          getenv("PDEIP_NO_TC_INTEGRATOR") == nullptr;
 }
 
-int launch_integrate_tensor(const IntegrateArgs& a, cudaStream_t st) {
+namespace itc {
+template <bool OD>
+static int launch_d_k(const IntegrateArgs& a, cudaStream_t st) {
   int* status = tensor_status_word();
   PDEIP_REQUIRE(status != nullptr, PDEIP_ERR_CUDA, "cannot allocate the tensor-path status word");
   status += 1;  // word 1: integrator (word 0: residual kernel)
   const int kp = (a.n_gaussian + 15) / 16 * 16;
   if (a.d == 8) {
-    if (kp == 16) return itc::launch8<16>(a, status, st);
-    if (kp == 32) return itc::launch8<32>(a, status, st);
-    if (kp == 48) return itc::launch8<48>(a, status, st);
-    return itc::launch8<64>(a, status, st);
+    if (kp == 16) return launch8<16, OD>(a, status, st);
+    if (kp == 32) return launch8<32, OD>(a, status, st);
+    if (kp == 48) return launch8<48, OD>(a, status, st);
+    return launch8<64, OD>(a, status, st);
   }
   if (a.d == 32) {
-    if (kp == 16) return itc::launch<32, 16>(a, status, st);
-    if (kp == 32) return itc::launch<32, 32>(a, status, st);
-    if (kp == 48) return itc::launch<32, 48>(a, status, st);
-    return itc::launch<32, 64>(a, status, st);
+    if (kp == 16) return launch<32, 16, OD>(a, status, st);
+    if (kp == 32) return launch<32, 32, OD>(a, status, st);
+    if (kp == 48) return launch<32, 48, OD>(a, status, st);
+    return launch<32, 64, OD>(a, status, st);
   }
-  if (kp == 16) return itc::launch<16, 16>(a, status, st);
-  if (kp == 32) return itc::launch<16, 32>(a, status, st);
-  if (kp == 48) return itc::launch<16, 48>(a, status, st);
-  return itc::launch<16, 64>(a, status, st);
+  if (kp == 16) return launch<16, 16, OD>(a, status, st);
+  if (kp == 32) return launch<16, 32, OD>(a, status, st);
+  if (kp == 48) return launch<16, 48, OD>(a, status, st);
+  return launch<16, 64, OD>(a, status, st);
 }
+}  // namespace itc
+
+int launch_integrate_tensor(const IntegrateArgs& a, cudaStream_t st) { return itc::launch_d_k<false>(a, st); }
+
+// true if an overdamped GMM call is served by K1-T-OD: d = 8, 16 or 32, 1..64 centres, Philox noise, AoS state with a
+// terminal-state output, every sample emitted, and either no trajectory or a BLOCK128 / TIME_SOA trajectory with the
+// drift (the arguments come on the UNIFORM schedule without tau0, pdeip_overdamped_integrate)
+bool overdamped_tensor_ok(const IntegrateArgs& a, int drift_kind) {
+  return drift_kind == PDEIP_DRIFT_GMM && (a.d == 8 || a.d == 16 || a.d == 32) && a.n_gaussian >= 1 &&
+         a.n_gaussian <= 64 && !a.noise && a.z_last && a.state_layout == PDEIP_LAYOUT_AOS && a.emit_every == 1 &&
+         a.emit_offset == 0 &&
+         (a.traj == nullptr ||
+          (a.emit_drift && (a.traj_layout == PDEIP_TRAJ_BLOCK128 || a.traj_layout == PDEIP_TRAJ_TIME_SOA))) &&
+         getenv("PDEIP_NO_TC_INTEGRATOR") == nullptr;
+}
+
+int launch_overdamped_tensor(const IntegrateArgs& a, cudaStream_t st) { return itc::launch_d_k<true>(a, st); }
 
 }  // namespace pdeip

@@ -130,7 +130,8 @@ def kl_integrate_model(z0: torch.Tensor, n_steps: int, dt: float, gamma: float, 
     return z_last, traj, tau
 
 
-def _od_buffers(x0, n_steps, noise, state_layout, traj_layout, want_traj, emit_every, emit_offset, emit_drift):
+def _od_buffers(x0, n_steps, noise, state_layout, traj_layout, want_traj, emit_every, emit_offset, emit_drift,
+                traj_out=None, x_last_out=None):
     """Checked inputs and the outputs of one K1-OD call: (x0, n, d, noise, x_last, traj|None)."""
     x0 = _f32(x0, "x0")
     if state_layout == L.LAYOUT_AOS:
@@ -148,7 +149,16 @@ def _od_buffers(x0, n_steps, noise, state_layout, traj_layout, want_traj, emit_e
                  L.TRAJ_TIME_SOA: (width, s_emit, n), L.TRAJ_BLOCK128: (s_emit, n // 128, width, 128)}[traj_layout]
         if traj_layout == L.TRAJ_BLOCK128 and n % 128:
             raise PdeipError(f"TRAJ_BLOCK128 needs n % 128 == 0, got n={n}")
-        traj = torch.empty(shape, device=x0.device, dtype=torch.float32)
+        if traj_out is not None:
+            if traj_out.numel() < n * s_emit * width:
+                raise PdeipError("traj_out too small")
+            traj = _f32(traj_out, "traj_out").view(-1)[: n * s_emit * width].view(shape)
+        else:
+            traj = torch.empty(shape, device=x0.device, dtype=torch.float32)
+    if x_last_out is not None:
+        if tuple(x_last_out.shape) != tuple(x0.shape) or _f32(x_last_out, "x_last_out") is not x_last_out:
+            raise PdeipError(f"x_last_out must be a contiguous {tuple(x0.shape)} tensor")
+        return x0, n, d, noise, x_last_out, traj
     return x0, n, d, noise, torch.empty_like(x0), traj
 
 
@@ -157,13 +167,16 @@ def overdamped_integrate(x0: torch.Tensor, n_steps: int, dt: float, drift_kind: 
                          noise: Optional[torch.Tensor] = None, seed: int = 0, particle_offset: int = 0,
                          step_offset: int = 0, state_layout: int = L.LAYOUT_AOS,
                          traj_layout: int = L.TRAJ_PARTICLE_MAJOR, want_traj: bool = True, emit_every: int = 1,
-                         emit_offset: int = 0, emit_drift: bool = False, path: int = L.PATH_FP32,
+                         emit_offset: int = 0, emit_drift: bool = False, path: int = L.PATH_FP32, *,
+                         traj_out: Optional[torch.Tensor] = None, x_last_out: Optional[torch.Tensor] = None,
                          ) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
     """pdeip_overdamped_integrate: n_steps overdamped Langevin steps x' = x - dt grad U(x) + sqrt(2 dt) xi.
     x0: [N,d] (AOS) or [d,N] (SOA).  noise: injected normals [N, n_steps, d], else Philox.  Returns (x_last,
-    traj|None); with emit_drift every trajectory sample is [x, grad U(x)] (2d components)."""
+    traj|None); with emit_drift every trajectory sample is [x, grad U(x)] (2d components).
+    path: PATH_TENSOR runs the GMM drift on tcgen05 inside its envelope (see pdeip.h).  traj_out / x_last_out:
+    buffers to write into (traj_out: at least the trajectory's size, viewed as its shape; x_last_out: x0's shape)."""
     x0, n, d, noise, x_last, traj = _od_buffers(x0, n_steps, noise, state_layout, traj_layout, want_traj, emit_every,
-                                                emit_offset, emit_drift)
+                                                emit_offset, emit_drift, traj_out, x_last_out)
     drift_params = _f32(drift_params, "drift_params", allow_none=True)
     _ops.overdamped_integrate(x0, x_last, traj, n, d, n_steps, float(dt), drift_kind, drift_params, n_gaussian,
                               float(sigma), noise, as_i64(seed), as_i64(particle_offset), step_offset, state_layout,

@@ -7,6 +7,14 @@ methods/consistency_instances/kinetic_fokker_planck.py:11-69 -> core/trainer.py:
 set [2d][S*Nc] and consumed immediately by the residual kernel, so the full [N, S, 2d] trajectory (54 GB at
 C3, 860 GB at C5) is never materialised.  Every emitted trajectory sample is a 0T point; the chunk's initial
 and terminal states are the boundary sets (the variant at GMM.py:144-156).
+
+HotPathConfig.dynamics = "overdamped" is the same iteration for the Fokker-Planck instance (dX = -grad U dt + sqrt(2) dW,
+fokker_planck_example_GMM.py): K1-OD emits each chunk as [x, grad U(x)] samples, which are directly an FP point set
+with DRIFT_IN_POINTS (SET_FP_0T), and the initial and terminal states are the FP boundary sets (SET_FP_BOUNDARY).
+
+Estimator: the 0T set is the time marginals on the uniform step grid, and the boundary sets come from the same
+ensemble as the 0T set.  The reference draws its 0T points at random times and its boundary samples independently;
+both variants estimate the same expectations.
 """
 from __future__ import annotations
 
@@ -20,23 +28,24 @@ from . import ops, parallel
 from .core.optimizer import AdamL2, OptState
 
 
-def integrator_wave(d: int, drift_kind: int, n_gaussian: int, path: int, sm_count: Optional[int] = None) -> int:
+def integrator_wave(d: int, drift_kind: int, n_gaussian: int, path: int, sm_count: Optional[int] = None, *,
+                    overdamped: bool = False) -> int:
     """Particles in one full wave of the production integrator grid (128 particles per CTA x CTAs per SM x SMs):
-    the tcgen05 GMM kernels run 8 (d = 8) / 3 (d = 16, 32) CTAs per SM, the fp32 kernel 4 (2 at d = 32)
-    (csrc/integrator_tc.cu, csrc/integrator.cu launch bounds)."""
+    the tcgen05 GMM kernels run 8 (d = 8) / 3 (d = 16, 32) CTAs per SM, their overdamped trajectory instances 6 (d = 8)
+    / 3 (d = 16, 32), the fp32 kernel 4 (2 at d = 32) (csrc/integrator_tc.cu, csrc/integrator.cu launch bounds)."""
     sms = sm_count if sm_count is not None else L.load().pdeip_sm_count()
     tensor = path == L.PATH_TENSOR and drift_kind == L.DRIFT_GMM and d in (8, 16, 32) and 1 <= n_gaussian <= 64
-    per_sm = (8 if d == 8 else 3) if tensor else (2 if d >= 32 else 4)
+    per_sm = ((6 if overdamped else 8) if d == 8 else 3) if tensor else (2 if d >= 32 else 4)
     return 128 * per_sm * sms
 
 
 def auto_chunk(d: int, n_steps: int, drift_kind: int, n_gaussian: int, path: int, emit_every: int = 1,
-               budget_bytes: float = 6.0e9, sm_count: Optional[int] = None) -> int:
-    """Largest whole number of integrator waves whose [x, v, grad U] trajectory fits `budget_bytes` (at least one wave):
-    no partially filled last wave, and a trajectory buffer far above the 126 MB L2."""
-    wave = integrator_wave(d, drift_kind, n_gaussian, path, sm_count)
+               budget_bytes: float = 6.0e9, sm_count: Optional[int] = None, *, overdamped: bool = False) -> int:
+    """Largest whole number of integrator waves whose [x, v, grad U] (overdamped: [x, grad U]) trajectory fits
+    `budget_bytes` (at least one wave): no partially filled last wave, and a trajectory buffer far above the 126 MB L2."""
+    wave = integrator_wave(d, drift_kind, n_gaussian, path, sm_count, overdamped=overdamped)
     s_emit = (n_steps + emit_every - 1) // emit_every
-    per_particle = 3 * d * s_emit * 4
+    per_particle = (2 if overdamped else 3) * d * s_emit * 4
     return wave * max(1, int(budget_bytes // (per_particle * wave)))
 
 
@@ -52,13 +61,21 @@ class HotPathConfig:
     chunk: int = 0  # particles per integrate -> residual round trip; 0 = auto_chunk(...)
     emit_every: int = 1
     path: int = L.PATH_FP32
+    dynamics: str = "kinetic"  # or "overdamped": K1-OD and the FP sets; the state is x [n, d] and gamma is ignored
 
 
 class HotPath:
     def __init__(self, cfg: HotPathConfig, model, params: Dict, drift_params: Optional[torch.Tensor],
                  true_grad: ops.TrueGrad, optimizer: Optional[AdamL2] = None, device="cuda"):
+        if cfg.dynamics not in ("kinetic", "overdamped"):
+            raise ValueError(f"unknown dynamics {cfg.dynamics!r}: 'kinetic' or 'overdamped'")
+        self.overdamped = cfg.dynamics == "overdamped"
+        if self.overdamped and cfg.drift_kind == L.DRIFT_MEANFIELD_TABLE:
+            raise ValueError("DRIFT_MEANFIELD_TABLE encodes the underdamped mean recursion; the overdamped dynamics "
+                             "do not take it")
         if cfg.chunk <= 0:
-            cfg.chunk = auto_chunk(cfg.d, cfg.n_steps, cfg.drift_kind, cfg.n_gaussian, cfg.path, cfg.emit_every)
+            cfg.chunk = auto_chunk(cfg.d, cfg.n_steps, cfg.drift_kind, cfg.n_gaussian, cfg.path, cfg.emit_every,
+                                   overdamped=self.overdamped)
         self.cfg, self.model, self.params = cfg, model, params
         self.drift_params, self.true_grad, self.optimizer = drift_params, true_grad, optimizer
         self.device = torch.device(device)
@@ -67,20 +84,25 @@ class HotPath:
         self.norms = torch.empty(2, device=self.device, dtype=torch.float32)
         s_emit = (cfg.n_steps + cfg.emit_every - 1) // cfg.emit_every
         self.s_emit = s_emit
-        # every sample carries [x, v, grad U(x)]: the integrator emits the drift it evaluates anyway
-        self.traj = torch.empty(3 * cfg.d * s_emit * cfg.chunk, device=self.device, dtype=torch.float32)
+        # every sample carries [x, v, grad U(x)] (overdamped: [x, grad U(x)]): the integrator emits the drift it
+        # evaluates anyway
+        self.width = (2 if self.overdamped else 3) * cfg.d  # floats per emitted sample
+        self.state = (1 if self.overdamped else 2) * cfg.d  # floats per state
+        self.traj = torch.empty(self.width * s_emit * cfg.chunk, device=self.device, dtype=torch.float32)
         self.true_in_points = ops.TrueGrad(L.DRIFT_IN_POINTS)
-        self.z_last = torch.empty((cfg.chunk, 2 * cfg.d), device=self.device, dtype=torch.float32)
-        self.z_last_full: Optional[torch.Tensor] = None  # [n, 2d] terminal states of all chunks (batched boundary sets)
-        self.z0_full: Optional[torch.Tensor] = None      # [n, 2d] device copy of the staged initial states (host-resident)
+        self.z_last = torch.empty((cfg.chunk, self.state), device=self.device, dtype=torch.float32)
+        self.z_last_full: Optional[torch.Tensor] = None  # [n, 2d] ([n, d] overdamped) terminal states of all chunks (batched boundary sets)
+        self.z0_full: Optional[torch.Tensor] = None      # [n, 2d] ([n, d]) device copy of the staged initial states (host-resident)
         # host-resident ensembles: two staging buffers and a copy stream, so that chunk k+1 crosses PCIe / NVLink-C2C
         # while chunk k is integrated
-        self.z_stage = [torch.empty((cfg.chunk, 2 * cfg.d), device=self.device, dtype=torch.float32) for _ in range(2)]
+        self.z_stage = [torch.empty((cfg.chunk, self.state), device=self.device, dtype=torch.float32) for _ in range(2)]
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.stage_ready = [torch.cuda.Event() for _ in range(2)]  # H2D of the buffer finished
         self.stage_free = [torch.cuda.Event() for _ in range(2)]   # last kernel reading the buffer finished
 
     def particle_steps(self, n: int) -> int:
+        if self.overdamped:
+            return n * self.cfg.n_steps  # S Euler-Maruyama steps per trajectory
         return n * (self.cfg.n_steps + 1)  # the reference does S+1 update_steps per trajectory
 
     def residual_evals(self, n: int) -> int:
@@ -106,8 +128,8 @@ class HotPath:
 
     def step(self, z0: torch.Tensor, seed: int, n_global: Optional[int] = None, particle_offset: int = 0,
              apply_optimizer: bool = True, phase_events: Optional[list] = None) -> Dict[str, torch.Tensor]:
-        """One iteration over the local ensemble z0 [n, 2d] (CUDA, or pinned host memory: then each chunk is
-        copied host->device inside the step).  n_global: ensemble size over all ranks (weights are 1/global
+        """One iteration over the local ensemble z0 [n, 2d] (overdamped: x0 [n, d]) (CUDA, or pinned host memory: then
+        each chunk is copied host->device inside the step).  n_global: ensemble size over all ranks (weights are 1/global
         counts so shards add up under one all-reduce).  phase_events: if a list, three CUDA events per chunk are
         appended to it (before the integrator, between integrator and 0T residual, after the 0T residual)."""
         c = self.cfg
@@ -130,9 +152,10 @@ class HotPath:
         # (bit-identical results).
         batched_boundary = n > c.chunk
         if batched_boundary and (self.z_last_full is None or self.z_last_full.shape[0] != n):
-            self.z_last_full = torch.empty((n, 2 * c.d), device=self.device, dtype=torch.float32)
+            self.z_last_full = torch.empty((n, self.state), device=self.device, dtype=torch.float32)
         if batched_boundary and staged and (self.z0_full is None or self.z0_full.shape[0] != n):
-            self.z0_full = torch.empty((n, 2 * c.d), device=self.device, dtype=torch.float32)
+            self.z0_full = torch.empty((n, self.state), device=self.device, dtype=torch.float32)
+        set_0T, set_b = (L.SET_FP_0T, L.SET_FP_BOUNDARY) if self.overdamped else (L.SET_KFP_0T, L.SET_KFP_BOUNDARY)
 
         def prefetch(k: int):  # H2D of chunk k into staging buffer k % 2 on the copy stream
             a, b = k * c.chunk, min(n, (k + 1) * c.chunk)
@@ -161,33 +184,40 @@ class HotPath:
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)] if phase_events is not None else None
             if ev:
                 ev[0].record()
-            z_last, traj, _ = ops.kl_integrate(
-                zc, c.n_steps, dt, c.gamma, c.drift_kind, drift_params, n_gaussian=c.n_gaussian, sigma=c.sigma,
-                seed=seed, particle_offset=particle_offset + lo,
-                traj_layout=L.TRAJ_BLOCK128 if blocked else L.TRAJ_TIME_SOA,
-                emit_every=c.emit_every, traj_out=self.traj,
-                z_last_out=self.z_last_full[lo:hi] if batched_boundary else self.z_last[:nc], emit_drift=True, path=c.path)
+            traj_layout = L.TRAJ_BLOCK128 if blocked else L.TRAJ_TIME_SOA
+            z_last_out = self.z_last_full[lo:hi] if batched_boundary else self.z_last[:nc]
+            if self.overdamped:
+                z_last, traj = ops.overdamped_integrate(
+                    zc, c.n_steps, dt, c.drift_kind, drift_params, n_gaussian=c.n_gaussian, sigma=c.sigma, seed=seed,
+                    particle_offset=particle_offset + lo, traj_layout=traj_layout, emit_every=c.emit_every,
+                    emit_drift=True, path=c.path, traj_out=self.traj, x_last_out=z_last_out)
+            else:
+                z_last, traj, _ = ops.kl_integrate(
+                    zc, c.n_steps, dt, c.gamma, c.drift_kind, drift_params, n_gaussian=c.n_gaussian, sigma=c.sigma,
+                    seed=seed, particle_offset=particle_offset + lo, traj_layout=traj_layout,
+                    emit_every=c.emit_every, traj_out=self.traj, z_last_out=z_last_out, emit_drift=True, path=c.path)
             if ev:
                 ev[1].record()
+            coef_0T = 0.0 if self.overdamped else c.gamma
             if blocked:
-                self.acc.accumulate(L.SET_KFP_0T, flat, traj.view(self.s_emit * nc // 128, 3 * c.d, 128), w_0T,
-                                    coef=c.gamma, layout=L.LAYOUT_BLOCK128, true_grad=self.true_in_points, path=c.path)
+                self.acc.accumulate(set_0T, flat, traj.view(self.s_emit * nc // 128, self.width, 128), w_0T,
+                                    coef=coef_0T, layout=L.LAYOUT_BLOCK128, true_grad=self.true_in_points, path=c.path)
             else:
-                self.acc.accumulate(L.SET_KFP_0T, flat, traj.view(3 * c.d, self.s_emit * nc), w_0T, coef=c.gamma,
+                self.acc.accumulate(set_0T, flat, traj.view(self.width, self.s_emit * nc), w_0T, coef=coef_0T,
                                     layout=L.LAYOUT_SOA, true_grad=self.true_in_points, path=c.path)
             if ev:
                 ev[2].record()
                 phase_events.append(ev)
             if not batched_boundary:
-                self.acc.accumulate(L.SET_KFP_BOUNDARY, flat, z_last, w_b, coef=2.0 / c.total_time, path=c.path)
-                self.acc.accumulate(L.SET_KFP_BOUNDARY, flat, zc, w_b, coef=-2.0 / c.total_time, path=c.path)
+                self.acc.accumulate(set_b, flat, z_last, w_b, coef=2.0 / c.total_time, path=c.path)
+                self.acc.accumulate(set_b, flat, zc, w_b, coef=-2.0 / c.total_time, path=c.path)
             if staged:
                 if batched_boundary:
                     self.z0_full[lo:hi].copy_(zc, non_blocking=True)  # device-to-device, before the buffer is released
                 self.stage_free[k % 2].record(main)
         if batched_boundary:
-            self.acc.accumulate(L.SET_KFP_BOUNDARY, flat, self.z_last_full, w_b, coef=2.0 / c.total_time, path=c.path)
-            self.acc.accumulate(L.SET_KFP_BOUNDARY, flat, self.z0_full if staged else z0, w_b, coef=-2.0 / c.total_time,
+            self.acc.accumulate(set_b, flat, self.z_last_full, w_b, coef=2.0 / c.total_time, path=c.path)
+            self.acc.accumulate(set_b, flat, self.z0_full if staged else z0, w_b, coef=-2.0 / c.total_time,
                                 path=c.path)
         sums, grad = self.acc.finalize()
         shard = parallel.Shard.current()
